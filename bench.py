@@ -2,8 +2,10 @@
 """bench.py -- the hot path of 2D-VQ-AE-2 on N B200s, with roofline and CPU baseline.
 
 Contract (one JSON line on stdout from rank 0):
-  python bench.py --gpus N --steps K --warmup W [--workload encode256|roundtrip512|slide]
+  python bench.py --gpus N --steps K --warmup W [--workload encode256|roundtrip512|slide] [--dump-outputs DIR]
   python bench.py --impl reference --gpus N ...    # the reference's own CPU implementation
+--dump-outputs DIR writes what the last timed step returned on rank 0 as DIR/<name>.npy (float32), so that
+two builds can be compared output for output on the same seeded inputs.
 For N > 1 launch with torch.distributed.run (one rank per GPU); patches shard by rank with no
 data-path collective (weak scaling); only the slide workload gathers code tiles with NCCL.
 
@@ -32,6 +34,9 @@ import time
 from pathlib import Path
 
 REPO = Path(__file__).resolve().parent
+# the benchmark writes nothing into the tree: its CPU legs import oracle/ modules that build() never
+# imported, and their bytecode would otherwise land in oracle/__pycache__
+sys.dont_write_bytecode = True
 for _p in (REPO / "2d-vq-ae-2_b200", REPO / "oracle"):
     if str(_p) not in sys.path:
         sys.path.insert(0, str(_p))
@@ -349,6 +354,23 @@ def device_patches(first: int, count: int, patch: int, dev) -> torch.Tensor:
     return out
 
 
+DUMP_MAX_ELEMS = 1 << 22        # per array: 16 MB of float32; at most two arrays per workload, 32 MB
+
+
+def host_outputs(outs, names) -> dict:
+    """float32 host copies of a step's outputs, taken before later steps reuse the graph's output
+    buffers.  An array larger than DUMP_MAX_ELEMS is stored as `<name>_sample`: the flattened array at
+    DUMP_MAX_ELEMS positions drawn from a fixed seed, the same positions in every run."""
+    outs = outs if isinstance(outs, tuple) else (outs,)
+    res = {}
+    for name, t in zip(names, outs, strict=True):
+        if t.numel() > DUMP_MAX_ELEMS:
+            pos = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0))
+            t, name = t.reshape(-1)[pos.to(t.device)], name + "_sample"
+        res[name] = t.float().cpu().numpy()
+    return res
+
+
 def run_gpu(args):
     rank, world, local = dist_env()
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (no CPU fallback)"
@@ -416,6 +438,7 @@ def run_gpu(args):
             g1.record()
             gather_ms.append((g0, g1))
             return code_map
+        out_names = ("code_map",)
         pool = [S.synthetic_patches_u8(B, PATCH, 42 + rank + 1000 * j).pin_memory() for j in range(4)]
         n_b = len(batches)
         h2d = sum(int(p.numel()) for _, p in batches)
@@ -448,6 +471,7 @@ def run_gpu(args):
         if args.workload == "encode256":
             def step_resident(i):
                 return encode_step(resident[i % 2])
+            out_names = ("codes",)
             streamer = StreamingEncoder(enc, dev, graphs=not args.no_graphs)
             h2d, d2h = int(B * PATCH * PATCH * 3), int(B * 32 * 32 * 8)
 
@@ -468,7 +492,8 @@ def run_gpu(args):
             roundtrip_step = captured(roundtrip)
 
             def step_resident(i):
-                return roundtrip_step(resident[i % 2])[1]
+                return roundtrip_step(resident[i % 2])
+            out_names = ("codes", "reconstruction")
             dev_in = [torch.empty_like(resident[0]) for _ in range(2)]
             host_idx = [torch.empty(B, 32, 32, dtype=torch.int64).pin_memory() for _ in range(2)]
             host_stat = torch.empty(2, dtype=torch.float32).pin_memory()
@@ -511,6 +536,7 @@ def run_gpu(args):
                    "on a side stream, D2H of int64 codes + reconstruction statistics every step")
 
     def timed(fn, steps, warmup):
+        """(max over ranks of the device time of `steps` calls of fn in ms, launches, last call's result)"""
         with torch.no_grad():
             for i in range(warmup):
                 fn(i)
@@ -519,20 +545,22 @@ def run_gpu(args):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
             for i in range(steps):
-                fn(i)
+                out = fn(i)
             e1.record()
             barrier()
             ms = e0.elapsed_time(e1)
             launches = E.launch_count() - l0
-        return allmax(ms), launches
+        return allmax(ms), launches, out
 
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     # at least three untimed steps: eager run, then one graph capture per input buffer
     warm = max(args.warmup, 3)
-    ms, launches = timed(step_resident, args.steps, warm)
+    ms, launches, last_out = timed(step_resident, args.steps, warm)
     clocks = sampler.stop() if rank == 0 else None
+    dumped = host_outputs(last_out, out_names) if args.dump_outputs and rank == 0 else None
+    del last_out
 
     with torch.no_grad():
         run_e2e(3 if args.workload == "slide" else warm)
@@ -558,7 +586,7 @@ def run_gpu(args):
                 continue
             vqae_b200.set_precision(model, prec)
             k = 3 if prec == "fp32" else max(3, args.steps // 2)
-            ms_p, _ = timed(step_resident, k, 2)
+            ms_p, _, _ = timed(step_resident, k, 2)
             modes[prec] = B * k / (ms_p * 1e-3)
         vqae_b200.set_precision(model, args.precision)
 
@@ -626,6 +654,11 @@ def run_gpu(args):
                     "workload": "as-shipped VQ-AE (n_down=4), encode+quantise+decode of 8 synthetic "
                                 "256x256x3 patches (16x16 codes)",
                     "seconds": min(ts), "patches_per_s": 8 / min(ts), "kind": cpu4.kind, "cores": cores}
+        if dumped is not None:
+            out_dir = Path(args.dump_outputs)
+            out_dir.mkdir(parents=True, exist_ok=True)
+            for name, arr in dumped.items():
+                np.save(out_dir / f"{name}.npy", arr)
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier()
@@ -644,7 +677,15 @@ def main():
                     help="launch every kernel of every step from the host instead of replaying CUDA graphs")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the side measurements (other precisions, config 2, CPU baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32; arrays above "
+                         f"{DUMP_MAX_ELEMS} elements as a seeded sample, <name>_sample.npy).  --impl b200 only: "
+                         "the reference leg times small CPU samples, not the inputs of the B200 path")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:
