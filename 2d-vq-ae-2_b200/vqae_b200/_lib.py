@@ -20,6 +20,7 @@ DT_F32, DT_BF16, DT_U8, DT_F16 = 0, 1, 2, 3
 QUANT_AUTO, QUANT_CUDA_CORE, QUANT_TENSOR_CORE = 0, 1, 2
 MODE_SAME, MODE_DOWN, MODE_UP = 0, 1, 2
 CONV_1x1, CONV_2x2S2, CONV_3x3_CIRC = 0, 1, 2
+STEM_OUT_EXACT, STEM_OUT_TENSOR_CORE = 0, 1
 
 
 class VqaeError(RuntimeError):
@@ -77,6 +78,9 @@ SIGNATURES = {
     "vqae_stem_in_f32": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i64, _i, _i, _i, _fp, _fp, _vp]),
     "vqae_stem_in": (_i, [_vp, _i, _i, _vp, _vp, _vp, _i, _i64, _i, _i, _i, _fp, _fp, _vp]),
     "vqae_stem_out_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i64, _i, _i, _i, _vp]),
+    "vqae_stem_out_u8_supported": (_i, [_i, _i, _i, _i]),
+    "vqae_stem_out_u8": (_i, [_vp, _vp, _vp, _fp, _fp, _vp, _i64, _i64, _i64, _i, _i64, _i, _i, _i, _i,
+                              _vp]),
     "vqae_conv_f32": (_i, [_i, _vp, _vp, _vp, _vp, _i64, _i, _i, _i, _i, _f, _i, _f, _f, _f, _vp]),
     "vqae_bicubic_up2_f32": (_i, [_vp, _vp, _i64, _i, _i, _i, _f, _vp]),
     "vqae_fixup_block_scratch_bytes": (_sz, [C.POINTER(FixupParams), _i64, _i, _i]),
@@ -92,6 +96,8 @@ SIGNATURES = {
     "vqae_quantize_tc_f32": (_i, [C.POINTER(QuantizerParams), _vp, _vp, _vp, _vp, _vp, _f, _vp,
                                   _vp, _vp, _sz, _i64, _i64, _vp]),
     "vqae_embed_codes_f32": (_i, [_vp, _i, _vp, _i, _i, _vp, _i, _i64, _i64, _vp]),
+    "vqae_embed_codemap_f32": (_i, [_vp, _i, _i64, _i64, _i, _i, _i64, _i64, _i64, _i64, _i64, _vp, _i,
+                                    _i, _vp, _vp]),
     "vqae_codemap_place_u8": (_i, [_vp, _i64, _i, _i, _i64, _i, _vp, _i64, _i64, _vp]),
     "vqae_codemap_place_i64": (_i, [_vp, _i64, _i, _i, _i64, _i, _vp, _i64, _i64, _vp]),
     "vqae_ema_scratch_bytes": (_sz, [_i64, _i, _i]),

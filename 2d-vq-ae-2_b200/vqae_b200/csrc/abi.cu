@@ -334,6 +334,29 @@ int vqae_stem_out_mma_f32(const float* x, const float* w_oihw, const float* bias
                         (cudaStream_t)stream);
 }
 
+int vqae_stem_out_u8_supported(int height, int width, int c_in, int kernel) {
+    if (kernel == VQAE_STEM_OUT_TENSOR_CORE) return stem_out_mma_supported(height, width, c_in) ? 1 : 0;
+    return kernel == VQAE_STEM_OUT_EXACT && height > 0 && width > 0 && c_in == 8 ? 1 : 0;
+}
+
+int vqae_stem_out_u8(const float* x, const float* w_oihw, const float* bias, const float* mean_host,
+                     const float* std_host, uint8_t* canvas, int64_t canvas_rows, int64_t canvas_cols,
+                     int64_t first_patch, int grid_cols, int64_t batch, int height, int width, int c_in,
+                     int kernel, void* stream) {
+    if (!x || !w_oihw || !bias) return VQAE_ERR_BAD_ARG;
+    U8Canvas cv{};
+    if (int rc = make_u8_canvas(canvas, canvas_rows, canvas_cols, first_patch, grid_cols, batch, height,
+                                width, mean_host, std_host, &cv))
+        return rc;
+    if (kernel == VQAE_STEM_OUT_EXACT)
+        return stem_out_u8(x, w_oihw, bias, cv, batch, height, width, c_in, (cudaStream_t)stream);
+    if (kernel != VQAE_STEM_OUT_TENSOR_CORE) return VQAE_ERR_BAD_ARG;
+    int sm_count = 0;
+    if (int rc = device_sm_count(&sm_count)) return rc;
+    return stem_out_mma_u8(x, w_oihw, bias, cv, batch, height, width, c_in, sm_count,
+                           (cudaStream_t)stream);
+}
+
 int vqae_front_fused_supported(int height, int width) {
     return front_fused_supported(height, width) ? 1 : 0;
 }
@@ -491,6 +514,14 @@ int vqae_embed_codes_f32(const void* indices, int idx_is_u8, const float* table,
                          void* stream) {
     return embed_codes_f32(indices, idx_is_u8, table, num_codes, c, out, out_layout, batch,
                            spatial, (cudaStream_t)stream);
+}
+
+int vqae_embed_codemap_f32(const void* code_map, int map_is_u8, int64_t map_rows, int64_t map_cols,
+                           int th, int tw, int64_t r0, int64_t c0, int64_t region_cols,
+                           int64_t first_patch, int64_t n, const float* table, int num_codes, int c,
+                           float* out, void* stream) {
+    return embed_codemap_f32(code_map, map_is_u8, map_rows, map_cols, th, tw, r0, c0, region_cols,
+                             first_patch, n, table, num_codes, c, out, (cudaStream_t)stream);
 }
 
 int vqae_codemap_place_u8(const int64_t* tiles, int64_t n_tiles, int th, int tw,

@@ -60,6 +60,28 @@ struct PreOp {
     }
 };
 
+// The uint8 output of out_stem, the exact inverse of the input normalisation (vqae_normalize_u8):
+// s_c = 255 std_c and o_c = 255 mean_c formed in fp32 on the host,
+//     u8 = min(max(rint(fma(v, s_c, o_c)), 0), 255)      round half to even; NaN -> 0 (fmaxf drops it)
+__device__ __forceinline__ uint8_t u8_store(float v, float s, float o) {
+    return (uint8_t)fminf(fmaxf(rintf(fmaf(v, s, o)), 0.0f), 255.0f);
+}
+
+// Where the uint8 form of out_stem writes: image b of the call is patch q = first_patch + b of a
+// canvas uint8 [canvas_rows, canvas_cols, 3] laid out as a grid of H x W patches with grid_cols
+// patches per row, i.e. at canvas pixel ((q / grid_cols) H, (q % grid_cols) W) -- the addressing
+// of codemap_place.  vec = 1: rows are 16-byte aligned (canvas_cols % 16 == 0, aligned base).
+struct U8Canvas {
+    uint8_t* canvas;
+    int64_t canvas_cols, first_patch;
+    int grid_cols, vec;
+    float s[3], o[3];
+};
+// host: validates the placement (VQAE_OK or VQAE_ERR_BAD_ARG) and fills the canvas descriptor
+int make_u8_canvas(uint8_t* canvas, int64_t canvas_rows, int64_t canvas_cols, int64_t first_patch,
+                   int grid_cols, int64_t B, int H, int W, const float* mean, const float* stdv,
+                   U8Canvas* cv);
+
 // Per-device caches: function attributes, occupancy results and scratch allocations belong to ONE
 // device; a process that drives several GPUs must not reuse them across devices.
 constexpr int kMaxDevices = 64;

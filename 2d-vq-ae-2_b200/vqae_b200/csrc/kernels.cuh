@@ -40,6 +40,8 @@ int stem_in_f32(const void* x, int x_dtype, int x_layout, const float* w, const 
                 const float* stdv, cudaStream_t stream);
 int stem_out_f32(const float* x, const float* w, const float* bias, float* out, int out_layout,
                  int64_t B, int H, int W, int c_in, cudaStream_t stream);
+int stem_out_u8(const float* x, const float* w, const float* bias, const U8Canvas& cv, int64_t B,
+                int H, int W, int c_in, cudaStream_t stream);
 
 // quantize.cu
 int quantizer_prepare_f32(const float* embed, int K, int D, const float* w_out,
@@ -57,6 +59,9 @@ int quantize_any(const vqae_quantizer_params* p, const void* x, int x_dtype, int
                  int64_t S, int kernel, cudaStream_t stream);
 int embed_codes_f32(const void* indices, int idx_is_u8, const float* table, int K, int C,
                     float* out, int out_layout, int64_t B, int64_t S, cudaStream_t stream);
+int embed_codemap_f32(const void* map, int map_is_u8, int64_t map_rows, int64_t map_cols, int th,
+                      int tw, int64_t r0, int64_t c0, int64_t region_cols, int64_t first_patch,
+                      int64_t n, const float* table, int K, int C, float* out, cudaStream_t stream);
 int codemap_place_u8(const int64_t* tiles, int64_t n_tiles, int th, int tw, int64_t first_patch,
                      int grid_cols, uint8_t* map, int64_t map_rows, int64_t map_cols,
                      cudaStream_t stream);
@@ -129,6 +134,8 @@ int stem_in_mma(const void* x, int x_dtype, int x_layout, const float* w, const 
                 int64_t B, int H, int W, int c_out, const float* mean, const float* stdv, int sm_count,
                 cudaStream_t stream);
 bool stem_out_mma_supported(int H, int W, int c_in);
+int stem_out_mma_u8(const float* x, const float* w, const float* bias, const U8Canvas& cv, int64_t B,
+                    int H, int W, int c_in, int sm_count, cudaStream_t stream);
 int stem_out_mma(const float* x, const float* w, const float* bias, float* out, int out_layout,
                  int64_t B, int H, int W, int c_in, int sm_count, cudaStream_t stream);
 

@@ -41,8 +41,9 @@ struct StemOutArgs {
     const float* x;          // NHWC fp32 [B,H,W,8]
     const float* w;          // OIHW [3,8,3,3]
     const float* bias;       // [3]
-    float* out;              // NCHW [B,3,H,W] or NHWC [B,H,W,3]
+    float* out;              // NCHW [B,3,H,W] or NHWC [B,H,W,3] (fp32 form)
     int n_tiles, H, W, tiles_x, tiles_per_img, nhwc_out;
+    U8Canvas cv;             // uint8 form
 };
 
 __device__ __forceinline__ void so_split2(float f0, float f1, uint32_t& hi, uint32_t& lo) {
@@ -53,6 +54,12 @@ __device__ __forceinline__ void so_split2(float f0, float f1, uint32_t& hi, uint
     lo = *reinterpret_cast<const uint32_t*>(&ll);
 }
 
+// U8: the de-normalising uint8 epilogue (u8_store) placing image b at patch first_patch + b of a
+// canvas.  A warp covers four 16-pixel row segments of a tile (48 bytes each, 16-byte aligned: tiles
+// start at multiples of 32 pixels = 96 bytes); their bytes are staged in the warp's 192 bytes of shared
+// memory and leave after its MMA steps as twelve 16-byte stores.  Everything up to the stored value is
+// the fp32 form's arithmetic.
+template <bool U8>
 __global__ void __launch_bounds__(SO_THREADS, 3)
 stem_out_mma_kernel(StemOutArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -124,6 +131,14 @@ stem_out_mma_kernel(StemOutArgs a) {
         __syncthreads();
         if (tile + (int)gridDim.x < a.n_tiles) fetch(tile + gridDim.x);
 
+        // u8: the tile's first canvas byte (32-bit patch arithmetic: first_patch + B < 2^31)
+        uint8_t* tile_dst = nullptr;
+        const int64_t row_bytes = a.cv.canvas_cols * 3;
+        if constexpr (U8) {
+            const int q = (int)a.cv.first_patch + img;
+            const int prow = q / a.cv.grid_cols, pcol = q - prow * a.cv.grid_cols;
+            tile_dst = a.cv.canvas + ((int64_t)prow * a.H + r0) * row_bytes + ((int64_t)pcol * a.W + c0) * 3;
+        }
         // ---- nine shifted K = 8 GEMM steps per M-tile (16 pixels of a row), two M-tiles per warp step
         const int lrow = (lane & 7) + ((lane >> 3) & 1) * 8;
 #pragma unroll 1
@@ -153,6 +168,25 @@ stem_out_mma_kernel(StemOutArgs a) {
                     mma_1688(d[u], h0, h1, bh[tap]);
                 }
             }
+            if constexpr (U8) {
+                // lane (g, t): t = 0 holds channels 0, 1 and t = 1 channel 2 of pixels g and g + 8;
+                // the warp's four 16-pixel segments of the tile go to its 192 staging bytes
+                uint8_t* st = smem + SO_SMEM + warp * 192 + (mt0 >> 4) * 96;
+                if (t < 2) {
+                    const float s0 = t ? a.cv.s[2] : a.cv.s[0], o0 = t ? a.cv.o[2] : a.cv.o[0];
+#pragma unroll
+                    for (int u = 0; u < 2; ++u) {
+                        uint8_t* sp = st + u * 48 + g * 3 + 2 * t;
+                        sp[0] = u8_store(d[u][0], s0, o0);
+                        sp[24] = u8_store(d[u][2], s0, o0);
+                        if (t == 0) {
+                            sp[1] = u8_store(d[u][1], a.cv.s[1], a.cv.o[1]);
+                            sp[25] = u8_store(d[u][3], a.cv.s[1], a.cv.o[1]);
+                        }
+                    }
+                }
+                continue;
+            }
 #pragma unroll
             for (int u = 0; u < 2; ++u) {
                 const int y = r0 + rr[u], x = c0 + cb[u] + g;
@@ -175,6 +209,30 @@ stem_out_mma_kernel(StemOutArgs a) {
                     }
                 }
             }
+        }
+        if constexpr (U8) {
+            // segment (j, u) of this warp is M-tile warp + 16 j + 8 u: tile row (mt >> 1), columns 16 (warp & 1)
+            __syncwarp();
+            const uint8_t* st = smem + SO_SMEM + warp * 192;
+            if (a.cv.vec) {
+                if (lane < 12) {
+                    const int seg = lane / 3, k = lane - 3 * seg;
+                    const int mt = warp + 16 * (seg >> 1) + 8 * (seg & 1);
+                    uint8_t* dst = tile_dst + (int64_t)(mt >> 1) * row_bytes + (mt & 1) * 48;
+                    reinterpret_cast<uint4*>(dst)[k] = reinterpret_cast<const uint4*>(st + seg * 48)[k];
+                }
+            } else {
+#pragma unroll
+                for (int pass = 0; pass < 2; ++pass) {
+                    const int seg = 2 * pass + (lane >> 4), px = lane & 15;
+                    const int mt = warp + 16 * pass + 8 * (lane >> 4);
+                    uint8_t* dst = tile_dst + (int64_t)(mt >> 1) * row_bytes + ((mt & 1) * 16 + px) * 3;
+                    dst[0] = st[seg * 48 + px * 3];
+                    dst[1] = st[seg * 48 + px * 3 + 1];
+                    dst[2] = st[seg * 48 + px * 3 + 2];
+                }
+            }
+            // the staging is rewritten only after the next tile's first barrier
         }
         __syncthreads();
     }
@@ -537,7 +595,23 @@ int stem_out_mma(const float* x, const float* w, const float* bias, float* out, 
     a.n_tiles = (int)nt;
     const int cap = sm_count * 3;
     const int grid = a.n_tiles < cap ? a.n_tiles : cap;
-    stem_out_mma_kernel<<<grid, SO_THREADS, SO_SMEM, stream>>>(a);
+    stem_out_mma_kernel<false><<<grid, SO_THREADS, SO_SMEM, stream>>>(a);
+    return check_launch();
+}
+
+int stem_out_mma_u8(const float* x, const float* w, const float* bias, const U8Canvas& cv, int64_t B,
+                    int H, int W, int c_in, int sm_count, cudaStream_t stream) {
+    if (!x || !w || !bias) return VQAE_ERR_BAD_ARG;
+    if (!stem_out_mma_supported(H, W, c_in)) return VQAE_ERR_UNSUPPORTED;
+    StemOutArgs a{};
+    a.x = x; a.w = w; a.bias = bias; a.out = nullptr; a.H = H; a.W = W; a.cv = cv;
+    a.tiles_x = W / SO_TW; a.tiles_per_img = (H / SO_TH) * a.tiles_x;
+    const int64_t nt = B * a.tiles_per_img;
+    if (nt > 0x7fffffff) return VQAE_ERR_UNSUPPORTED;
+    a.n_tiles = (int)nt;
+    const int cap = sm_count * 3;
+    const int grid = a.n_tiles < cap ? a.n_tiles : cap;
+    stem_out_mma_kernel<true><<<grid, SO_THREADS, SO_SMEM + SO_WARPS * 192, stream>>>(a);
     return check_launch();
 }
 

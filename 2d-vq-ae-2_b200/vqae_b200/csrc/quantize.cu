@@ -297,6 +297,32 @@ embed_codes_kernel(const void* __restrict__ indices, const float* __restrict__ t
     }
 }
 
+// embed_codes on a window of a stored code map: patch t of the call is region patch first_patch + t
+// (region_cols patches per region row, region origin (r0, c0) in patches), code (y, x) of it sits at
+// map[((r0 + pr) th + y) map_cols + (c0 + pc) tw + x].  Thread j of image row blockIdx.y writes float4
+// j of the patch's NHWC rows: consecutive threads read consecutive codes of one map row (each code
+// once per C / 4 threads) and write consecutive output float4s.
+template <bool U8>
+__global__ void __launch_bounds__(256)
+embed_codemap_kernel(const void* __restrict__ map, int64_t map_cols, int th, int tw, int64_t r0,
+                     int64_t c0, int64_t region_cols, int64_t first_patch, int64_t n,
+                     const float4* __restrict__ tab, int K, int c4n, float4* __restrict__ out) {
+    const int per_patch = th * tw * c4n;
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= per_patch) return;
+    const int pix = j / c4n, c4 = j - pix * c4n;
+    const int y = pix / tw, x = pix - y * tw;
+    for (int64_t t = blockIdx.y; t < n; t += gridDim.y) {
+        const int64_t q = first_patch + t;
+        const int64_t pr = q / region_cols, pc = q - pr * region_cols;
+        const int64_t m = ((r0 + pr) * th + y) * map_cols + (c0 + pc) * tw + x;
+        int64_t k = U8 ? (int64_t) reinterpret_cast<const uint8_t*>(map)[m]
+                       : reinterpret_cast<const int64_t*>(map)[m];
+        k = k < 0 ? 0 : (k >= K ? K - 1 : k);                   // embed_codes_kernel's clamping
+        out[t * per_patch + j] = __ldg(tab + k * c4n + c4);
+    }
+}
+
 template <typename MapT>
 __global__ void __launch_bounds__(256)
 codemap_place_kernel(const int64_t* __restrict__ tiles, int64_t total, int th, int tw,
@@ -443,6 +469,29 @@ int embed_codes_f32(const void* indices, int idx_is_u8, const float* table, int 
     else
         embed_codes_kernel<false><<<grid, 256, 0, stream>>>(indices, table, K, C, out, out_layout,
                                                             B * S, S);
+    return check_launch();
+}
+
+int embed_codemap_f32(const void* map, int map_is_u8, int64_t map_rows, int64_t map_cols, int th,
+                      int tw, int64_t r0, int64_t c0, int64_t region_cols, int64_t first_patch,
+                      int64_t n, const float* table, int K, int C, float* out, cudaStream_t stream) {
+    if (!map || !table || !out || map_rows <= 0 || map_cols <= 0 || th <= 0 || tw <= 0 || n <= 0 ||
+        region_cols <= 0 || K <= 0 || C <= 0 || r0 < 0 || c0 < 0 || first_patch < 0)
+        return VQAE_ERR_BAD_ARG;
+    const int64_t last = first_patch + n - 1;               // the window must lie inside the map
+    if ((r0 + last / region_cols + 1) * th > map_rows || (c0 + region_cols) * tw > map_cols)
+        return VQAE_ERR_BAD_ARG;
+    if (C % 4 != 0 || (int64_t)th * tw * (C / 4) > 0x7fffffff) return VQAE_ERR_UNSUPPORTED;
+    const int c4n = C / 4;
+    const dim3 grid(ceil_div_u((int64_t)th * tw * c4n, 256), (unsigned)(n < 65535 ? n : 65535));
+    const float4* tab = reinterpret_cast<const float4*>(table);
+    float4* o4 = reinterpret_cast<float4*>(out);
+    if (map_is_u8)
+        embed_codemap_kernel<true><<<grid, 256, 0, stream>>>(map, map_cols, th, tw, r0, c0, region_cols,
+                                                             first_patch, n, tab, K, c4n, o4);
+    else
+        embed_codemap_kernel<false><<<grid, 256, 0, stream>>>(map, map_cols, th, tw, r0, c0, region_cols,
+                                                              first_patch, n, tab, K, c4n, o4);
     return check_launch();
 }
 

@@ -3,6 +3,7 @@
 //                    (conf/transforms/camelyon16_transforms.yaml:1-23, transforms/normalize.yaml)
 //   stem_in_f32    : Encoder.in_stem  (vq_ae/model.py:141,198)  3x3, zero pad, bias, 3 -> 8
 //   stem_out_f32   : Decoder.out_stem (vq_ae/model.py:291)      3x3, zero pad, bias, 8 -> 3
+//   stem_out_u8    : the same with de-normalised uint8 RGB output placed into a slide canvas
 #include <cuda_fp16.h>
 
 #include "common.cuh"
@@ -247,11 +248,14 @@ stem_in_tiled_kernel(const void* __restrict__ xv, const float* __restrict__ w_oi
     }
 }
 
-template <int CIN>
+// U8: the de-normalising uint8 epilogue (u8_store, common.cuh) placing image b at patch
+// first_patch + b of a canvas; a warp's 32 pixels (one row segment when W % 32 == 0) are staged in
+// shared memory and leave as six 16-byte stores.  The arithmetic up to the stored value is shared.
+template <int CIN, bool U8>
 __global__ void __launch_bounds__(256)
 stem_out_kernel(const float* __restrict__ x, const float* __restrict__ w_oihw,
                 const float* __restrict__ bias, float* __restrict__ out, int out_layout,
-                int64_t npix, int H, int W) {
+                int64_t npix, int H, int W, U8Canvas cv) {
     __shared__ float ws[9 * CIN][3];  // [(ky*3+kx)*CIN + c][o]
     __shared__ float bs[3];
     for (int i = threadIdx.x; i < 3 * CIN * 9; i += blockDim.x) {
@@ -295,6 +299,27 @@ stem_out_kernel(const float* __restrict__ x, const float* __restrict__ w_oihw,
                 }
             }
         }
+    }
+    if constexpr (U8) {
+        __shared__ __align__(16) uint8_t st[8][96];                 // one 32-pixel segment per warp
+        const int q = (int)cv.first_patch + (int)b;                 // first_patch + B < 2^31
+        const int prow = q / cv.grid_cols, pcol = q - prow * cv.grid_cols;
+        uint8_t* dst = cv.canvas + (((int64_t)prow * H + y) * cv.canvas_cols + (int64_t)pcol * W + xx) * 3;
+        const uint8_t r8 = u8_store(a0, cv.s[0], cv.o[0]), g8 = u8_store(a1, cv.s[1], cv.o[1]),
+                      b8 = u8_store(a2, cv.s[2], cv.o[2]);
+        if (!cv.vec) {
+            dst[0] = r8; dst[1] = g8; dst[2] = b8;
+            return;
+        }
+        // vec: W % 32 == 0, so a warp's 32 pixels are one 96-byte segment of an image row (and
+        // npix % 32 == 0: no warp is cut by the early return above)
+        const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
+        st[wp][lane * 3] = r8; st[wp][lane * 3 + 1] = g8; st[wp][lane * 3 + 2] = b8;
+        __syncwarp();
+        uint8_t* seg = dst - lane * 3;                               // the segment's first byte
+        if (lane < 6)
+            reinterpret_cast<uint4*>(seg)[lane] = reinterpret_cast<const uint4*>(st[wp])[lane];
+        return;
     }
     if (out_layout == VQAE_LAYOUT_NHWC) {
         out[p * 3 + 0] = a0;
@@ -366,8 +391,40 @@ int stem_out_f32(const float* x, const float* w, const float* bias, float* out, 
     if (!x || !w || !bias || !out || B <= 0 || H <= 0 || W <= 0) return VQAE_ERR_BAD_ARG;
     if (c_in != 8) return VQAE_ERR_UNSUPPORTED;
     const int64_t npix = B * H * W;
-    stem_out_kernel<8><<<ceil_div_u(npix, 256), 256, 0, stream>>>(x, w, bias, out, out_layout,
-                                                                  npix, H, W);
+    stem_out_kernel<8, false><<<ceil_div_u(npix, 256), 256, 0, stream>>>(x, w, bias, out, out_layout,
+                                                                         npix, H, W, U8Canvas{});
+    return check_launch();
+}
+
+int make_u8_canvas(uint8_t* canvas, int64_t canvas_rows, int64_t canvas_cols, int64_t first_patch,
+                   int grid_cols, int64_t B, int H, int W, const float* mean, const float* stdv,
+                   U8Canvas* cv) {
+    if (!canvas || !mean || !stdv || B <= 0 || H <= 0 || W <= 0 || canvas_rows <= 0 ||
+        canvas_cols <= 0 || grid_cols <= 0 || first_patch < 0)
+        return VQAE_ERR_BAD_ARG;
+    const int64_t last = first_patch + B - 1;
+    if ((int64_t)grid_cols * W > canvas_cols || (last / grid_cols + 1) * H > canvas_rows)
+        return VQAE_ERR_BAD_ARG;
+    if (last > 0x7fffffff) return VQAE_ERR_UNSUPPORTED;           // patch indices are 32-bit in the kernels
+    cv->canvas = canvas;
+    cv->canvas_cols = canvas_cols;
+    cv->first_patch = first_patch;
+    cv->grid_cols = grid_cols;
+    cv->vec = W % 32 == 0 && canvas_cols % 16 == 0 && (reinterpret_cast<uintptr_t>(canvas) & 15u) == 0;
+    for (int c = 0; c < 3; ++c) {
+        cv->s[c] = 255.0f * stdv[c];           // the fp32 products of the normalisation
+        cv->o[c] = 255.0f * mean[c];
+    }
+    return VQAE_OK;
+}
+
+int stem_out_u8(const float* x, const float* w, const float* bias, const U8Canvas& cv, int64_t B,
+                int H, int W, int c_in, cudaStream_t stream) {
+    if (!x || !w || !bias) return VQAE_ERR_BAD_ARG;
+    if (c_in != 8) return VQAE_ERR_UNSUPPORTED;
+    const int64_t npix = B * H * W;
+    stem_out_kernel<8, true><<<ceil_div_u(npix, 256), 256, 0, stream>>>(x, w, bias, nullptr,
+                                                                        VQAE_LAYOUT_NHWC, npix, H, W, cv);
     return check_launch();
 }
 

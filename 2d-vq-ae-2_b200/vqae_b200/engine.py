@@ -764,6 +764,33 @@ def stem_out(x_nhwc: Tensor, weight: Tensor, bias: Tensor, channels_last: bool,
     return out.permute(0, 3, 1, 2) if channels_last else out
 
 
+def stem_out_u8(x_nhwc: Tensor, weight: Tensor, bias: Tensor, canvas: Tensor, first_patch: int = 0,
+                grid_cols: int = 1, mean=None, std=None, precision: str = "fp32") -> Tensor:
+    """NHWC fp32 [B,H,W,8] -> uint8 RGB pixels, de-normalised with ``mean`` / ``std`` (default: the
+    CAMELYON16 constants of ``Encoder.encode``) and rounded half to even (vqae_stem_out_u8).  Image b
+    lands at patch ``first_patch + b`` of ``canvas`` (contiguous uint8 [rows, cols, 3], a grid of H x W
+    patches with ``grid_cols`` per row); ``grid_cols = 1, first_patch = 0`` on a [B*H, W, 3] view is a
+    plain [B,H,W,3] batch.  Kernel choice as in ``stem_out``: "fp32" the exact CUDA-core kernel,
+    other precisions the split-operand tensor-core kernel where it tiles the image."""
+    lib = L.load()
+    require_cuda(x_nhwc, "stem_out_u8")
+    x_nhwc = _as_stream(x_nhwc, False).contiguous()
+    b, h, wd, c = x_nhwc.shape
+    if canvas.dtype != torch.uint8 or canvas.dim() != 3 or canvas.shape[2] != 3 or \
+            not canvas.is_contiguous() or canvas.device != x_nhwc.device:
+        raise ValueError("canvas must be a contiguous uint8 [rows, cols, 3] tensor on the input's device")
+    w = weight.detach().float().contiguous()
+    bi = bias.detach().float().contiguous()
+    kernel = L.STEM_OUT_EXACT
+    if precision != "fp32" and lib.vqae_stem_out_u8_supported(h, wd, c, L.STEM_OUT_TENSOR_CORE):
+        kernel = L.STEM_OUT_TENSOR_CORE
+    L.check(lib.vqae_stem_out_u8(_ptr(x_nhwc), _ptr(w), _ptr(bi), L.f3(mean or CAMELYON16_MEAN),
+                                 L.f3(std or CAMELYON16_STD), _ptr(canvas), canvas.shape[0],
+                                 canvas.shape[1], first_patch, grid_cols, b, h, wd, c,
+                                 kernel, _stream(x_nhwc.device)), "vqae_stem_out_u8")
+    return canvas
+
+
 def normalize_u8(img: Tensor, mean=CAMELYON16_MEAN, std=CAMELYON16_STD,
                  channels_last: bool = False) -> Tensor:
     """u8 [B,H,W,3] -> fp32 [B,3,H,W]."""
@@ -897,6 +924,26 @@ def embed_codes(pq: PackedQuantizer, idx: Tensor, out_nhwc: bool, batch: int, sp
                                      _ptr(out), L.LAYOUT_NHWC if out_nhwc else L.LAYOUT_NCHW,
                                      batch, spatial, _stream(idx.device)),
             "vqae_embed_codes_f32")
+    return out
+
+
+def embed_codemap(pq: PackedQuantizer, code_map: Tensor, code_hw: Tuple[int, int], r0: int, c0: int,
+                  region_cols: int, first_patch: int, n: int) -> Tensor:
+    """``embed_codes`` of n code tiles gathered straight from a stored map (vqae_embed_codemap_f32):
+    code_map uint8 / int64 [rows*th, cols*tw]; patch t is region patch ``first_patch + t`` of the region
+    with origin (r0, c0) (in patches) and ``region_cols`` patches per row.  Returns NHWC fp32
+    [n, th, tw, C]."""
+    lib = L.load()
+    require_cuda(code_map, "embed_codemap")
+    if code_map.dtype not in (torch.uint8, torch.int64) or code_map.dim() != 2:
+        raise ValueError("embed_codemap reads a 2-D uint8 or int64 code map")
+    code_map = code_map.contiguous()
+    th, tw = code_hw
+    out = torch.empty(n, th, tw, pq.c, dtype=torch.float32, device=code_map.device)
+    L.check(lib.vqae_embed_codemap_f32(_ptr(code_map), int(code_map.dtype == torch.uint8),
+                                       code_map.shape[0], code_map.shape[1], th, tw, r0, c0, region_cols,
+                                       first_patch, n, _ptr(pq.table), pq.k, pq.c, _ptr(out),
+                                       _stream(code_map.device)), "vqae_embed_codemap_f32")
     return out
 
 

@@ -17,6 +17,7 @@ import numpy as np
 import torch
 
 from . import engine as E
+from . import plan as P
 from .graphs import CapturedStep
 from .plan import resolve_precision
 from .sharding import gather_code_tiles, shard_range, slide_grid  # noqa: F401
@@ -244,6 +245,59 @@ class StreamingEncoder:
             i += 1
         for oslot in pending:
             yield result(oslot)
+
+
+@torch.no_grad()
+def decompress_region(model, code_map: torch.Tensor, code_hw: Tuple[int, int],
+                      region: Optional[Tuple[int, int, int, int]] = None, batch: int = 256, mean=None,
+                      std=None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The inverse of ``compress_slide``: decode a stored code map (or a region of it) to uint8 RGB
+    pixels on the map's device.
+
+    ``code_map`` [rows*th, cols*tw] of th x tw code tiles (``code_hw``), uint8 or int64 as stored, or any
+    other integer / bool dtype that ``cast_to_lowest_dtype`` / ``np.load`` produce (widened to int64
+    once).  ``region = (r0, c0, nr, nc)`` in patches, default the whole map.  Patches are gathered from
+    the map, decoded and written into the [nr*H, nc*W, 3] result (``out`` if given) by the kernels,
+    at most ``batch`` patches per step; H, W = th, tw times 2 per 'up' block of the decoder.  Each patch
+    is decoded on its own, exactly like the model decodes a tile.  Reads ``model.encoder.vq_layers[0]``
+    and ``model.decoder`` only, so an ``accelerate()``-d reference model works too.  ``mean`` / ``std``:
+    the normalisation to undo (default CAMELYON16, as in ``compress_slide``)."""
+    vq, dec = model.encoder.vq_layers[0], model.decoder
+    P.check_u8_decoder(dec, "decompress_region")
+    E.require_cuda(code_map, "decompress_region")
+    if code_map.dim() != 2:
+        raise ValueError(f"code_map must be 2-D, got shape {tuple(code_map.shape)}")
+    if code_map.dtype not in (torch.uint8, torch.int64):
+        if code_map.dtype.is_floating_point or code_map.dtype.is_complex:
+            raise ValueError(f"code_map must hold integer codes, got {code_map.dtype}")
+        code_map = code_map.long()
+    th, tw = (int(v) for v in code_hw)
+    if th <= 0 or tw <= 0 or code_map.shape[0] % th or code_map.shape[1] % tw:
+        raise ValueError(f"code map {tuple(code_map.shape)} is not a grid of {th} x {tw} code tiles")
+    rows, cols = code_map.shape[0] // th, code_map.shape[1] // tw
+    r0, c0, nr, nc = (int(v) for v in (region if region is not None else (0, 0, rows, cols)))
+    if r0 < 0 or c0 < 0 or nr <= 0 or nc <= 0 or r0 + nr > rows or c0 + nc > cols:
+        raise ValueError(f"region {(r0, c0, nr, nc)} leaves the {rows} x {cols} patch grid")
+    if batch <= 0:
+        raise ValueError("batch must be positive")
+    pq = P.packed_quantizer(vq)
+    if code_map.dtype != torch.uint8 or pq.k < 256:
+        win = code_map[r0 * th:(r0 + nr) * th, c0 * tw:(c0 + nc) * tw]
+        if bool(((win < 0) | (win >= pq.k)).any()):
+            raise ValueError(f"code map holds codes outside [0, {pq.k})")
+    f = P.patch_scale(dec)
+    shape = (nr * th * f, nc * tw * f, 3)
+    if out is None:
+        out = torch.empty(shape, dtype=torch.uint8, device=code_map.device)
+    elif tuple(out.shape) != shape or out.dtype != torch.uint8 or out.device != code_map.device \
+            or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous uint8 tensor of shape {shape} on {code_map.device}")
+    total = nr * nc
+    for first in range(0, total, batch):
+        n = min(batch, total - first)
+        enc = E.embed_codemap(pq, code_map, (th, tw), r0, c0, nc, first, n)
+        P.decoder_forward_u8(dec, enc, mean, std, out, first, nc)
+    return out
 
 
 def tiles_to_map(tiles_u8: torch.Tensor, grid: Tuple[int, int]) -> torch.Tensor:

@@ -160,6 +160,15 @@ class VQAE(nn.Module):
         enc = self.encoder.vq_layers[0].decode_codes(indices, channels_last)
         return self.decoder((enc,))
 
+    @torch.no_grad()
+    def decode_codes_u8(self, indices: Tensor, mean=None, std=None) -> Tensor:
+        """Decompress stored codes [B,h,w] (int64 or uint8, CUDA) to uint8 RGB pixels [B,H,W,3]: the
+        decoder of ``decode_codes`` with the normalisation undone inside out_stem's kernel,
+        ``rint(v * 255 std_c + 255 mean_c)`` clamped to [0, 255].  ``mean`` / ``std`` default to the
+        CAMELYON16 constants, as in ``Encoder.encode``, so ``encoder.encode(decode_codes_u8(idx))`` is a
+        round trip.  Precision follows the decoder (``set_precision``, ``torch.autocast``)."""
+        return P.decode_codes_u8(self.encoder.vq_layers[0], self.decoder, indices, mean, std)
+
     def transfer_batch_to_device(self, batch: Tensor, device: torch.device,
                                  dataloader_idx: int = 0) -> Tensor:
         return batch.to(device, non_blocking=True, memory_format=torch.channels_last)

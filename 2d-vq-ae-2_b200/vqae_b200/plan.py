@@ -394,6 +394,52 @@ def decoder_forward(dec, xs: Sequence[Tensor]) -> Tensor:
     return E.stem_out(h, dec.out_stem.weight, dec.out_stem.bias, cl, precision)
 
 
+def check_u8_decoder(dec, who: str = "decoder_forward_u8") -> None:
+    """The uint8 output exists for the fused single-level plan of Fixup decoders (conf/model/vq_ae.yaml)."""
+    _check_single_level(len(dec.up_layers), dec.shortcut_layers, who)
+    if any(M.is_mbconv(m) for m in dec.modules()):
+        raise NotImplementedError(f"{who}: decoders with MBConv blocks have no uint8 output")
+    if dec.training:
+        raise RuntimeError("Decoder: training-mode forward is outside the B200 inference "
+                           "path; call .eval()")
+
+
+def patch_scale(dec) -> int:
+    """Pixels per code along each axis: x2 per 'up' block of the decoder."""
+    return 2 ** sum(E.infer_block_mode(b) == "up" for b in flat_blocks(dec.up_layers))
+
+
+def decoder_forward_u8(dec, enc_nhwc: Tensor, mean=None, std=None, canvas: Optional[Tensor] = None,
+                       first_patch: int = 0, grid_cols: int = 1) -> Tensor:
+    """The single-level plan of ``decoder_forward`` on NHWC fp32 [B,h,w,C] encodings with out_stem's
+    uint8 epilogue (E.stem_out_u8): the same blocks and kernels as the float output, then de-normalised
+    RGB pixels placed as patches first_patch .. first_patch + B - 1 of ``canvas`` (grid_cols per row).
+    ``canvas=None`` returns a fresh uint8 [B,H,W,3]."""
+    check_u8_decoder(dec)
+    E.require_cuda(enc_nhwc, "Decoder.forward")
+    precision = resolve_precision(dec)
+    h = _plan(dec).run(flat_blocks(dec.post_enc_layers) + flat_blocks(dec.up_layers), enc_nhwc.contiguous(),
+                       precision)
+    b, hh, ww, _ = h.shape
+    if canvas is None:
+        canvas = torch.empty(b, hh, ww, 3, dtype=torch.uint8, device=h.device)
+        E.stem_out_u8(h, dec.out_stem.weight, dec.out_stem.bias, canvas.view(b * hh, ww, 3), 0, 1,
+                      mean, std, precision)
+        return canvas
+    return E.stem_out_u8(h, dec.out_stem.weight, dec.out_stem.bias, canvas, first_patch, grid_cols,
+                         mean, std, precision)
+
+
+def decode_codes_u8(vq, dec, indices: Tensor, mean=None, std=None) -> Tensor:
+    """embed_code -> proj_out -> Decoder -> uint8 RGB [B,H,W,3] for stored codes [B,h,w] (int64 / uint8)."""
+    check_u8_decoder(dec, "decode_codes_u8")
+    E.require_cuda(indices, "decode_codes_u8")
+    pq = packed_quantizer(vq)
+    b, h, w = indices.shape
+    enc = E.embed_codes(pq, indices.reshape(-1), True, b, h * w).view(b, h, w, pq.c)
+    return decoder_forward_u8(dec, enc, mean, std)
+
+
 def block_forward(block, inp: Tensor) -> Tensor:
     """One PreActFixupResBlock on an NCHW / channels_last tensor (conv_block.py:196-216)."""
     if block.training:

@@ -193,6 +193,26 @@ int vqae_stem_out_mma_supported(int height, int width, int c_in);
 int vqae_stem_out_mma_f32(const float* x, const float* w_oihw, const float* bias, float* out,
                           int out_layout, int64_t batch, int height, int width, int c_in,
                           void* stream);
+/* out_stem with the uint8 output of a decoded slide: the exact inverse of vqae_normalize_u8,
+ *     u8 = min(max(rint(fma(v, 255 std_c, 255 mean_c)), 0), 255)     (round half to even; NaN -> 0)
+ * with v the fp32 value the fp32 form of the same kernel stores and the two products formed in fp32
+ * on the host.  Image b of the batch is written as patch q = first_patch + b of a canvas uint8
+ * [canvas_rows, canvas_cols, 3] (NHWC RGB, the layout vqae_stem_in reads) holding a grid of
+ * height x width patches, grid_cols per row: at canvas pixel ((q / grid_cols) height,
+ * (q % grid_cols) width) -- the addressing of vqae_codemap_place_u8.  grid_cols = 1 and
+ * first_patch = 0 on a [batch * height, width, 3] canvas is the plain [B,H,W,3] batch.
+ * kernel: VQAE_STEM_OUT_EXACT (the CUDA-core kernel of vqae_stem_out_f32, bit-identical values before
+ * the conversion) or VQAE_STEM_OUT_TENSOR_CORE (that of vqae_stem_out_mma_f32; height % 16 == 0,
+ * width % 32 == 0).  Rows leave as 16-byte stores when width % 32 == 0, canvas_cols % 16 == 0 and
+ * the canvas is 16-byte aligned.  x NHWC fp32 [B,H,W,c_in], c_in == 8; mean/std: host float[3].
+ * VQAE_ERR_BAD_ARG for a null pointer, a non-positive extent or a placement outside the canvas,
+ * checked before anything is launched; VQAE_ERR_UNSUPPORTED when first_patch + batch > 2^31.       */
+enum { VQAE_STEM_OUT_EXACT = 0, VQAE_STEM_OUT_TENSOR_CORE = 1 };
+int vqae_stem_out_u8_supported(int height, int width, int c_in, int kernel);
+int vqae_stem_out_u8(const float* x, const float* w_oihw, const float* bias, const float* mean_host,
+                     const float* std_host, uint8_t* canvas, int64_t canvas_rows, int64_t canvas_cols,
+                     int64_t first_patch, int grid_cols, int64_t batch, int height, int width, int c_in,
+                     int kernel, void* stream);
 /* The encoder's FRONT END in one launch (csrc/mma_front.cu): in_stem (with the u8 normalisation of
  * vqae_stem_in) + the C = 8 'same' block + the 'down' block 8 -> 16 of the first DownBlock
  * (model.py:141,144-148,198-199) -- the input image is read once, the 16-channel half-resolution
@@ -364,6 +384,17 @@ int vqae_quantize_tc_f32(const vqae_quantizer_params* p, const float* x, float* 
 int vqae_embed_codes_f32(const void* indices, int idx_is_u8, const float* table, int num_codes,
                          int c, float* out, int out_layout, int64_t batch, int64_t spatial,
                          void* stream);
+
+/* vqae_embed_codes_f32 straight out of a stored code map: code_map u8 (map_is_u8 = 1) or int64
+ * [map_rows, map_cols] made of th x tw code tiles; a region of region_cols patches per row starts at
+ * patch (r0, c0); patch t = 0 .. n-1 of the call is region patch first_patch + t, i.e. map patch
+ * (r0 + (first_patch + t) / region_cols, c0 + (first_patch + t) % region_cols).  out: NHWC fp32
+ * [n, th, tw, c] = table[code] (codes clamped to [0, num_codes) like vqae_embed_codes_f32).
+ * VQAE_ERR_BAD_ARG for a null pointer, a non-positive extent or a window outside the map.      */
+int vqae_embed_codemap_f32(const void* code_map, int map_is_u8, int64_t map_rows, int64_t map_cols,
+                           int th, int tw, int64_t r0, int64_t c0, int64_t region_cols,
+                           int64_t first_patch, int64_t n, const float* table, int num_codes, int c,
+                           float* out, void* stream);
 
 /* ---- a-X  code-map placement (scripts/extract_embeddings/extract_embeddings.py:47-59,75-89) -
  * Places n_tiles [th,tw] int64 code tiles at (row*th, col*tw) of a u8 map [rows*th, cols*tw];
