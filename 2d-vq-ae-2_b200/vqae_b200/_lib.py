@@ -109,6 +109,9 @@ SIGNATURES = {
     "vqae_pointwise_conv_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _i, _i, _i, _i, _vp]),
     "vqae_depthwise_conv_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _i, _i, _vp]),
     "vqae_se_gate_f32": (_i, [_vp, _i64, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
+    "vqae_quality_u8_scratch_bytes": (_sz, [_i64, _i, _i]),
+    "vqae_quality_u8": (_i, [_vp, _i64, _i64, _i64, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _i64, _i64,
+                             _i64, _i, _i, _vp, _vp, _vp, _sz, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -538,4 +538,18 @@ int vqae_codemap_place_i64(const int64_t* tiles, int64_t n_tiles, int th, int tw
                              map_cols, (cudaStream_t)stream);
 }
 
+size_t vqae_quality_u8_scratch_bytes(int64_t batch, int height, int width) {
+    return quality_u8_scratch_bytes(batch, height, width);
+}
+
+int vqae_quality_u8(const uint8_t* ref, int64_t ref_rows, int64_t ref_cols, int64_t ref_r0, int64_t ref_c0,
+                    int64_t ref_region_cols, int64_t ref_first, const uint8_t* rec, int64_t rec_rows,
+                    int64_t rec_cols, int64_t rec_r0, int64_t rec_c0, int64_t rec_region_cols,
+                    int64_t rec_first, int64_t batch, int height, int width, int64_t* sse, double* ssim,
+                    void* scratch, size_t scratch_bytes, void* stream) {
+    return quality_u8(ref, ref_rows, ref_cols, ref_r0, ref_c0, ref_region_cols, ref_first, rec, rec_rows,
+                      rec_cols, rec_r0, rec_c0, rec_region_cols, rec_first, batch, height, width, sse, ssim,
+                      scratch, scratch_bytes, (cudaStream_t)stream);
+}
+
 }  // extern "C"

@@ -174,4 +174,12 @@ int down_block_tc(const void* x, void* out, int io_dtype, const void* w_packed,
                   const float* scalars8, int64_t B, int H, int W, int CI, int sm_count,
                   cudaStream_t stream);
 
+// quality.cu (per-patch SSE and SSIM of two uint8 RGB images)
+size_t quality_u8_scratch_bytes(int64_t batch, int H, int W);
+int quality_u8(const uint8_t* ref, int64_t ref_rows, int64_t ref_cols, int64_t ref_r0, int64_t ref_c0,
+               int64_t ref_rc, int64_t ref_first, const uint8_t* rec, int64_t rec_rows, int64_t rec_cols,
+               int64_t rec_r0, int64_t rec_c0, int64_t rec_rc, int64_t rec_first, int64_t batch, int H,
+               int W, int64_t* sse, double* ssim, void* scratch, size_t scratch_bytes,
+               cudaStream_t stream);
+
 }  // namespace vqae

@@ -973,6 +973,31 @@ def codemap_place_i64(tiles: Tensor, first_patch: int, grid_cols: int, code_map:
                                        _stream(tiles.device)), "vqae_codemap_place_i64")
 
 
+def quality_u8(ref_canvas: Tensor, ref_addr: Tuple[int, int, int, int], rec_canvas: Tensor,
+               rec_addr: Tuple[int, int, int, int], batch: int, h: int, w: int) -> Tuple[Tensor, Tensor]:
+    """Per-patch SSE (int64 [batch, 3]) and SSIM (float64 [batch]) of ``batch`` h x w patches of two
+    uint8 RGB canvases (vqae_quality_u8).  Each canvas is a contiguous uint8 [rows, cols, 3] tensor
+    holding a grid of h x w patches; ``addr = (r0, c0, region_cols, first)`` puts patch t of the call at
+    grid position (r0 + (first + t) // region_cols, c0 + (first + t) % region_cols).  ``(0, 0, 1, 0)``
+    on a [batch*h, w, 3] view is a plain batch."""
+    lib = L.load()
+    require_cuda(ref_canvas, "quality_u8")
+    for cv in (ref_canvas, rec_canvas):
+        if cv.dtype != torch.uint8 or cv.dim() != 3 or cv.shape[2] != 3 or not cv.is_contiguous() or \
+                cv.device != ref_canvas.device:
+            raise ValueError("quality_u8 reads contiguous uint8 [rows, cols, 3] canvases on one device")
+    dev = ref_canvas.device
+    sse = torch.empty(batch, 3, dtype=torch.int64, device=dev)
+    ssim = torch.empty(batch, dtype=torch.float64, device=dev)
+    ws = workspace(dev, lib.vqae_quality_u8_scratch_bytes(batch, h, w))
+    (ar0, ac0, arc, afirst), (br0, bc0, brc, bfirst) = ref_addr, rec_addr
+    L.check(lib.vqae_quality_u8(_ptr(ref_canvas), ref_canvas.shape[0], ref_canvas.shape[1], ar0, ac0, arc,
+                                afirst, _ptr(rec_canvas), rec_canvas.shape[0], rec_canvas.shape[1], br0, bc0,
+                                brc, bfirst, batch, h, w, _ptr(sse), _ptr(ssim), _ptr(ws), ws.numel(),
+                                _stream(dev)), "vqae_quality_u8")
+    return sse, ssim
+
+
 # ---- f-4: training-mode codebook maintenance, level sums -------------------------------------------
 def add_nhwc(a: Tensor, b: Tensor, out: Optional[Tensor] = None) -> Tensor:
     """a + b for two contiguous fp32 tensors of one shape (the level sums of model.py:208, 283-288)."""

@@ -10,6 +10,7 @@ advanced indexing.
 """
 from __future__ import annotations
 
+import math
 from pathlib import Path
 from typing import Dict, Iterable, Iterator, Optional, Sequence, Tuple
 
@@ -20,6 +21,7 @@ from . import engine as E
 from . import plan as P
 from .graphs import CapturedStep
 from .plan import resolve_precision
+from .quality import ReconstructionQuality, check_u8_patches, reconstruction_quality
 from .sharding import gather_code_tiles, shard_range, slide_grid  # noqa: F401
 
 
@@ -247,24 +249,13 @@ class StreamingEncoder:
             yield result(oslot)
 
 
-@torch.no_grad()
-def decompress_region(model, code_map: torch.Tensor, code_hw: Tuple[int, int],
-                      region: Optional[Tuple[int, int, int, int]] = None, batch: int = 256, mean=None,
-                      std=None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """The inverse of ``compress_slide``: decode a stored code map (or a region of it) to uint8 RGB
-    pixels on the map's device.
-
-    ``code_map`` [rows*th, cols*tw] of th x tw code tiles (``code_hw``), uint8 or int64 as stored, or any
-    other integer / bool dtype that ``cast_to_lowest_dtype`` / ``np.load`` produce (widened to int64
-    once).  ``region = (r0, c0, nr, nc)`` in patches, default the whole map.  Patches are gathered from
-    the map, decoded and written into the [nr*H, nc*W, 3] result (``out`` if given) by the kernels,
-    at most ``batch`` patches per step; H, W = th, tw times 2 per 'up' block of the decoder.  Each patch
-    is decoded on its own, exactly like the model decodes a tile.  Reads ``model.encoder.vq_layers[0]``
-    and ``model.decoder`` only, so an ``accelerate()``-d reference model works too.  ``mean`` / ``std``:
-    the normalisation to undo (default CAMELYON16, as in ``compress_slide``)."""
+def _region_plan(model, code_map: torch.Tensor, code_hw: Tuple[int, int],
+                 region: Optional[Tuple[int, int, int, int]], batch: int, who: str):
+    """The argument checks of ``decompress_region`` / ``score_region``: returns (packed quantiser,
+    decoder, code map (uint8 or int64), (th, tw), (rows, cols), (r0, c0, nr, nc), patch scale)."""
     vq, dec = model.encoder.vq_layers[0], model.decoder
-    P.check_u8_decoder(dec, "decompress_region")
-    E.require_cuda(code_map, "decompress_region")
+    P.check_u8_decoder(dec, who)
+    E.require_cuda(code_map, who)
     if code_map.dim() != 2:
         raise ValueError(f"code_map must be 2-D, got shape {tuple(code_map.shape)}")
     if code_map.dtype not in (torch.uint8, torch.int64):
@@ -285,7 +276,26 @@ def decompress_region(model, code_map: torch.Tensor, code_hw: Tuple[int, int],
         win = code_map[r0 * th:(r0 + nr) * th, c0 * tw:(c0 + nc) * tw]
         if bool(((win < 0) | (win >= pq.k)).any()):
             raise ValueError(f"code map holds codes outside [0, {pq.k})")
-    f = P.patch_scale(dec)
+    return pq, dec, code_map, (th, tw), (rows, cols), (r0, c0, nr, nc), P.patch_scale(dec)
+
+
+@torch.no_grad()
+def decompress_region(model, code_map: torch.Tensor, code_hw: Tuple[int, int],
+                      region: Optional[Tuple[int, int, int, int]] = None, batch: int = 256, mean=None,
+                      std=None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The inverse of ``compress_slide``: decode a stored code map (or a region of it) to uint8 RGB
+    pixels on the map's device.
+
+    ``code_map`` [rows*th, cols*tw] of th x tw code tiles (``code_hw``), uint8 or int64 as stored, or any
+    other integer / bool dtype that ``cast_to_lowest_dtype`` / ``np.load`` produce (widened to int64
+    once).  ``region = (r0, c0, nr, nc)`` in patches, default the whole map.  Patches are gathered from
+    the map, decoded and written into the [nr*H, nc*W, 3] result (``out`` if given) by the kernels,
+    at most ``batch`` patches per step; H, W = th, tw times 2 per 'up' block of the decoder.  Each patch
+    is decoded on its own, exactly like the model decodes a tile.  Reads ``model.encoder.vq_layers[0]``
+    and ``model.decoder`` only, so an ``accelerate()``-d reference model works too.  ``mean`` / ``std``:
+    the normalisation to undo (default CAMELYON16, as in ``compress_slide``)."""
+    pq, dec, code_map, (th, tw), _, (r0, c0, nr, nc), f = _region_plan(model, code_map, code_hw, region,
+                                                                       batch, "decompress_region")
     shape = (nr * th * f, nc * tw * f, 3)
     if out is None:
         out = torch.empty(shape, dtype=torch.uint8, device=code_map.device)
@@ -298,6 +308,73 @@ def decompress_region(model, code_map: torch.Tensor, code_hw: Tuple[int, int],
         enc = E.embed_codemap(pq, code_map, (th, tw), r0, c0, nc, first, n)
         P.decoder_forward_u8(dec, enc, mean, std, out, first, nc)
     return out
+
+
+@torch.no_grad()
+def compress_slide_scored(model, batches: Iterable[Tuple[int, torch.Tensor]], grid: Tuple[int, int],
+                          code_hw: Tuple[int, int], device: torch.device, mean=None, std=None
+                          ) -> Tuple[torch.Tensor, ReconstructionQuality]:
+    """``compress_slide`` that also scores what the stored codes decode to.  For every
+    (first_patch_index, uint8 [B,H,W,3] tiles) batch: encode, place the codes (the returned map is the
+    one ``compress_slide`` returns), decode the batch's codes to uint8 pixels (``decode_codes_u8``) and
+    score them against the tiles (``reconstruction_quality``).  The decoded pixels live for one batch.
+    Returns ``(code_map, quality)``; ``quality`` holds per-patch maps ``sse`` [rows, cols, 3] and
+    ``ssim`` [rows, cols] in slide order (patches no batch covers keep sse 0 and ssim NaN).  Reads
+    ``model.encoder`` and ``model.decoder``; ``mean`` / ``std`` as in ``compress_slide``."""
+    enc_mod, dec = model.encoder, model.decoder
+    _check_u8_codes(enc_mod)
+    P.check_u8_decoder(dec, "compress_slide_scored")
+    rows, cols = grid
+    th, tw = code_hw
+    f = P.patch_scale(dec)
+    hw = (th * f, tw * f)
+    code_map = torch.zeros(rows * th, cols * tw, dtype=torch.uint8, device=device)
+    sse = torch.zeros(rows * cols, 3, dtype=torch.int64, device=device)
+    ssim = torch.full((rows * cols,), math.nan, dtype=torch.float64, device=device)
+    vq = enc_mod.vq_layers[0]
+    for first_patch, patches in batches:
+        check_u8_patches(patches, "compress_slide_scored: a patch batch")
+        if tuple(patches.shape[1:3]) != hw:
+            raise ValueError(f"patches of {tuple(patches.shape[1:3])} pixels do not decode from "
+                             f"{th} x {tw} code tiles ({hw[0]} x {hw[1]} pixels)")
+        x = patches.to(device, non_blocking=True)
+        idx = encode_patches(enc_mod, x, mean, std)
+        E.codemap_place(idx, first_patch, cols, code_map)
+        q = reconstruction_quality(x.contiguous(), P.decode_codes_u8(vq, dec, idx, mean, std))
+        sse[first_patch:first_patch + len(idx)] = q.sse
+        ssim[first_patch:first_patch + len(idx)] = q.ssim
+    return code_map, ReconstructionQuality(sse.view(rows, cols, 3), ssim.view(rows, cols), hw)
+
+
+@torch.no_grad()
+def score_region(model, code_map: torch.Tensor, code_hw: Tuple[int, int], slide_u8: torch.Tensor,
+                 region: Optional[Tuple[int, int, int, int]] = None, batch: int = 256, mean=None,
+                 std=None) -> ReconstructionQuality:
+    """Score a stored code map against the original slide: decode the region (as ``decompress_region``
+    does, at most ``batch`` patches per step into one reused buffer) and compare each decoded batch with
+    the slide's pixels in place.  ``slide_u8``: contiguous uint8 [rows*H, cols*W, 3] on the map's device,
+    the whole slide the map was made from.  Returns per-patch maps ``sse`` [nr, nc, 3] and ``ssim``
+    [nr, nc] of the region ``(r0, c0, nr, nc)`` (default the whole map).  Argument checks as in
+    ``decompress_region``."""
+    pq, dec, code_map, (th, tw), (rows, cols), (r0, c0, nr, nc), f = _region_plan(
+        model, code_map, code_hw, region, batch, "score_region")
+    h, w = th * f, tw * f
+    shape = (rows * h, cols * w, 3)
+    if not isinstance(slide_u8, torch.Tensor) or tuple(slide_u8.shape) != shape or \
+            slide_u8.dtype != torch.uint8 or slide_u8.device != code_map.device or not slide_u8.is_contiguous():
+        raise ValueError(f"slide_u8 must be a contiguous uint8 tensor of shape {shape} on {code_map.device}")
+    total = nr * nc
+    sse = torch.empty(total, 3, dtype=torch.int64, device=code_map.device)
+    ssim = torch.empty(total, dtype=torch.float64, device=code_map.device)
+    buf = torch.empty(min(batch, total) * h, w, 3, dtype=torch.uint8, device=code_map.device)
+    for first in range(0, total, batch):
+        n = min(batch, total - first)
+        enc = E.embed_codemap(pq, code_map, (th, tw), r0, c0, nc, first, n)
+        rec = buf[:n * h]
+        P.decoder_forward_u8(dec, enc, mean, std, rec, 0, 1)
+        sse[first:first + n], ssim[first:first + n] = E.quality_u8(slide_u8, (r0, c0, nc, first), rec,
+                                                                   (0, 0, 1, 0), n, h, w)
+    return ReconstructionQuality(sse.view(nr, nc, 3), ssim.view(nr, nc), (h, w))
 
 
 def tiles_to_map(tiles_u8: torch.Tensor, grid: Tuple[int, int]) -> torch.Tensor:

@@ -409,6 +409,34 @@ int vqae_codemap_place_i64(const int64_t* tiles, int64_t n_tiles, int th, int tw
                            int64_t first_patch, int grid_cols, int64_t* map, int64_t map_rows,
                            int64_t map_cols, void* stream);
 
+/* ---- reconstruction quality of uint8 RGB patches (csrc/quality.cu) ---------------------------
+ * The reference publishes reconstruction MSE (README.md:35,40) and validation MSE / PSNR / SSIM per
+ * codebook size (scripts/extract_validation_metrics/results.md:3-6, eval.py:13-45, torchmetrics).
+ * This call scores an original patch x against its reconstruction y, both uint8 H x W x 3:
+ *   sse[b, c]  = sum over the patch of (x - y)^2 in channel c, exact (integer arithmetic), int64;
+ *   ssim[b]    = mean over the 3 channels and the (H - 10)(W - 10) valid window positions (no padding)
+ *                of (2 mu_x mu_y + C1)(2 s_xy + C2) / ((mu_x^2 + mu_y^2 + C1)(s_xx + s_yy + C2)),
+ *                11 x 11 Gaussian window (sigma 1.5, the 11 taps normalised to sum 1 in float64 and
+ *                rounded once to fp32), population moments, C1 = (0.01 * 255)^2, C2 = (0.03 * 255)^2;
+ *                float64, moments accumulated in float64.
+ * This is skimage.metrics.structural_similarity(gaussian_weights=True, sigma=1.5,
+ * use_sample_covariance=False, data_range=255, channel_axis=-1).  Each input is a canvas uint8
+ * [rows, cols, 3] holding a grid of height x width patches; patch t of the call sits at grid position
+ * (r0 + (first + t) / region_cols, c0 + (first + t) % region_cols) -- the addressing of
+ * vqae_embed_codemap_f32; region_cols = 1 on a [batch * height, width, 3] canvas is a plain batch.
+ * Results depend on each patch's pixels only (not on its position in the batch, the batch size or the
+ * grid): bitwise reproducible.  Checked before anything is launched: VQAE_ERR_BAD_ARG for a null
+ * pointer, a non-positive extent or a placement outside either canvas; VQAE_ERR_UNSUPPORTED for
+ * height or width < 11 or first + batch > 2^31; VQAE_ERR_SCRATCH when scratch is missing or smaller
+ * than vqae_quality_u8_scratch_bytes (0 for an unsupported shape).                                */
+size_t vqae_quality_u8_scratch_bytes(int64_t batch, int height, int width);
+int vqae_quality_u8(const uint8_t* ref, int64_t ref_rows, int64_t ref_cols, int64_t ref_r0, int64_t ref_c0,
+                    int64_t ref_region_cols, int64_t ref_first,
+                    const uint8_t* rec, int64_t rec_rows, int64_t rec_cols, int64_t rec_r0, int64_t rec_c0,
+                    int64_t rec_region_cols, int64_t rec_first,
+                    int64_t batch, int height, int width, int64_t* sse, double* ssim,
+                    void* scratch, size_t scratch_bytes, void* stream);
+
 /* ---- f-4  training-mode codebook maintenance (layers/vq.py:47-94) -----------------------------
  * EMAVectorQuantizer._update_ema / _init_ema without the N x K one-hot matrix of the reference:
  *   vqae_ema_accumulate_f32   counts[k] = #{n : idx[n] = k},  dw[k,:] = sum of z[n,:] over those n
