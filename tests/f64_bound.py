@@ -122,32 +122,38 @@ def round_f16(x: Bounded) -> Bounded:
 
 
 def conv(x: Bounded, w: Tensor, r: Rounding, stride: int = 1, pad: Optional[str] = None,
-         w_abs: float = 0.0) -> Bounded:
+         w_abs: float = 0.0, into: Optional[Bounded] = None) -> Bounded:
     """conv2d without bias (``pad``: None, "circular" (the 'same' branch conv) or "zero" (the stems)).
-    ``r.emulate``: the operand is rounded to fp16 first, and ``w`` (fp32, as packed) too."""
+    ``r.emulate``: the operand is rounded to fp16 first, and ``w`` (fp32, as packed) too.
+    ``into``: the products accumulate onto this value in the same fp32 accumulator (one more term of
+    the sum, whose magnitude joins the accumulation error)."""
     if r.emulate:
         x = round_f16(x)
         w = _f16(w)
     w = w.double()
     aw = w.abs()
     m = x.mag()
-    k = r.terms * w.shape[1] * w.shape[2] * w.shape[3]
+    k = r.terms * w.shape[1] * w.shape[2] * w.shape[3] + (into is not None)
     carried = x.e + r.act * m + r.act_abs
     y = F.conv2d(_pad(x.v, pad), w, stride=stride)
     e = F.conv2d(_pad(carried, pad), aw, stride=stride) + \
         F.conv2d(_pad(m, pad), (r.w + gamma(k, r.acc)) * aw + w_abs, stride=stride)
+    if into is not None:
+        y = y + into.v
+        e = e + into.e + gamma(k, r.acc) * into.mag()
     return Bounded(y, e)
 
 
-def pre_act(x: Bounded, a: float, b: Optional[float], elu: bool = True) -> Bounded:
-    """elu(x + a) + b (the Fixup pre-activation; ``elu=False``: x + a, the skip path)."""
+def pre_act(x: Bounded, a: float, b: Optional[float], elu: bool = True, a_mag: float = 0.0) -> Bounded:
+    """elu(x + a) + b (the Fixup pre-activation; ``elu=False``: x + a, the skip path).  ``a_mag``: the
+    kernel folds further terms of this size into ``a`` (the resident kernel's running bias4)."""
     s = x.v + a
     if not elu:
         return Bounded(s, x.e + U_EW * s.abs())
     v = O.elu(s) + (b or 0.0)
     # the fp16 kernels form elu(x + a) + b as x + (a + b) or exp2(x log2e + a log2e) + (b - 1)
     # (mma_common.cuh:33-35): roundings of a few ulps of |a| and |b| as well
-    return Bounded(v, x.e + U_EW * (s.abs() + v.abs() + abs(a) + abs(b or 0.0)) + EW_ABS)
+    return Bounded(v, x.e + U_EW * (s.abs() + v.abs() + abs(a) + a_mag + abs(b or 0.0)) + EW_ABS)
 
 
 def affine(x: Bounded, scale: float, bias: float) -> Bounded:
@@ -187,20 +193,26 @@ def bicubic(x: Bounded, r: Rounding) -> Bounded:
     return Bounded(O.bicubic_up2(x.v), bicubic_abs(carried) + gamma(16 * r.terms, r.acc) * bicubic_abs(m))
 
 
-def fixup_block(x: Tensor, p: Mapping[str, Tensor], r: Rounding, interp: Optional[Rounding] = None,
-                fold_scale: bool = False, w_abs: Tuple[float, float, float] = (0.0, 0.0, 0.0)
-                ) -> Bounded:
-    """O.fixup_block in float64 with its bound.  ``r``: the rounding of every conv; ``interp``: that of
-    the 'up' interpolation (default ``r``); ``fold_scale``: the kernel multiplies branch_conv3 by the
-    Fixup scale at pack time (rounded with the weights), otherwise it scales the accumulator.  An 'up'
-    block is evaluated as the kernels do: both 1x1 ResizeConv2D convs at low resolution, then the
-    upsample (they commute; |W| and the |taps| commute too, so the bound holds for either order)."""
+def fixup_block(x, p: Mapping[str, Tensor], r: Rounding, interp: Optional[Rounding] = None,
+                fold_scale: bool = False, w_abs: Tuple[float, float, float] = (0.0, 0.0, 0.0),
+                residual_in_acc: bool = False, cum_mag: float = 0.0) -> Bounded:
+    """O.fixup_block in float64 with its bound.  ``x``: a Tensor (exact) or a ``Bounded`` that carries
+    an input error in.  ``r``: the rounding of every conv; ``interp``: that of the 'up' interpolation
+    (default ``r``); ``fold_scale``: the kernel multiplies branch_conv3 by the Fixup scale at pack time
+    (rounded with the weights), otherwise it scales the accumulator.  An 'up' block is evaluated as the
+    kernels do: both 1x1 ResizeConv2D convs at low resolution, then the upsample (they commute; |W| and
+    the |taps| commute too, so the bound holds for either order).
+
+    ``residual_in_acc`` (tc_resident.cu, a 'same' block with ``fold_scale``): branch_conv3 accumulates
+    straight into the fp32 residual, so the residual add is one more accumulation term, charged as
+    gamma(C + 1) (|R| + |W3s| conv |V|); bias4 joins a running sum that the kernel folds into the next
+    block's bias1a and adds at the store (``cum_mag``: a bound on |that sum| when this block starts)."""
     f = lambda k: float(p[k])                                         # noqa: E731
     w1, w2, w3 = p["branch_conv1.weight"], p["branch_conv2.weight"], p["branch_conv3.weight"]
     k2 = w2.shape[-1]
     interp = interp or r
-    x = exact(x)
-    h = pre_act(x, f("bias1a"), f("bias1b"))
+    x = x if isinstance(x, Bounded) else exact(x)
+    h = pre_act(x, f("bias1a"), f("bias1b"), a_mag=cum_mag)
     h = conv(h, w1, r, w_abs=w_abs[0])
     h = pre_act(h, f("bias2a"), f("bias2b"))
     if k2 == 3:
@@ -213,6 +225,11 @@ def fixup_block(x: Tensor, p: Mapping[str, Tensor], r: Rounding, interp: Optiona
     scale = float(p["scale"])
     if fold_scale:
         w3s = w3.float() * torch.tensor(scale, dtype=torch.float32)      # pack.cu: fp32 product
+        if residual_in_acc:
+            h = conv(h, w3s, r, w_abs=w_abs[2], into=x)
+            # the accumulator holds R = y - cum, so |R| <= |y| + |cum| joins the accumulation term
+            h = Bounded(h.v, h.e + gamma(r.terms * w3.shape[1] + 1, r.acc) * cum_mag)
+            return affine(h, 1.0, f("bias4"))
         h = affine(conv(h, w3s, r, w_abs=w_abs[2]), 1.0, f("bias4"))
     else:
         h = affine(conv(h, w3, r, w_abs=w_abs[2]), scale, f("bias4"))
@@ -227,6 +244,16 @@ def fixup_block(x: Tensor, p: Mapping[str, Tensor], r: Rounding, interp: Optiona
     else:
         s = conv(s, ws, r, w_abs=w_abs[2])
     return add(h, affine(s, 1.0, f("bias1d")))
+
+
+def resident_carry(y: Tensor, bias4s) -> Tuple[Bounded, float]:
+    """The input of block k + 1 of an image-resident run (tc_resident.cu) as the stored output y_k of
+    the k-block run, and a bound on |cum_k|, the running fp32 sum of the bias4 of those k blocks
+    (float64 sum plus one rounding per add).  The kernel holds R_k = y_k - cum_k in tensor memory; y_k
+    is R_k + cum_k rounded once: carried error 2^-24 (|y_k| + |cum_k|)."""
+    cum = abs(sum(bias4s)) + len(bias4s) * 2.0 ** -24 * sum(abs(b) for b in bias4s)
+    y = y.double()
+    return Bounded(y, 2.0 ** -24 * (y.abs() + cum)), cum
 
 
 def stem(x: Bounded, w: Tensor, bias: Tensor, r: Rounding, w_abs: float = 0.0) -> Bounded:
