@@ -112,6 +112,12 @@ SIGNATURES = {
     "vqae_quality_u8_scratch_bytes": (_sz, [_i64, _i, _i]),
     "vqae_quality_u8": (_i, [_vp, _i64, _i64, _i64, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _i64, _i64,
                              _i64, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    "vqae_codemap_histogram": (_i, [_vp, _i, _i64, _i64, _i64, _i64, _i64, _i64, _i, _vp, _vp]),
+    "vqae_codemap_pack_scratch_bytes": (_sz, [_i64, _i, _i]),
+    "vqae_codemap_pack_worst_bytes": (_i64, [_i64, _i, _i]),
+    "vqae_codemap_pack": (_i, [_vp, _i, _i64, _i64, _i, _i, _vp, _i, _i, _vp, _vp, _i64, _vp, _sz, _vp]),
+    "vqae_codemap_unpack": (_i, [_vp, _i64, _vp, _vp, _i64, _i64, _i, _i, _vp, _i, _i, _i64, _i64, _i64, _i64,
+                                 _vp, _i, _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

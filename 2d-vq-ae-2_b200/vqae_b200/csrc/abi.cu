@@ -552,4 +552,34 @@ int vqae_quality_u8(const uint8_t* ref, int64_t ref_rows, int64_t ref_cols, int6
                       scratch, scratch_bytes, (cudaStream_t)stream);
 }
 
+int vqae_codemap_histogram(const void* map, int map_is_u8, int64_t map_rows, int64_t map_cols, int64_t r0,
+                           int64_t c0, int64_t nr, int64_t nc, int num_codes, int64_t* counts, void* stream) {
+    return codemap_histogram(map, map_is_u8, map_rows, map_cols, r0, c0, nr, nc, num_codes, counts,
+                             (cudaStream_t)stream);
+}
+
+size_t vqae_codemap_pack_scratch_bytes(int64_t n_patches, int th, int tw) {
+    return codemap_pack_scratch_bytes(n_patches, th, tw);
+}
+
+int64_t vqae_codemap_pack_worst_bytes(int64_t n_patches, int th, int tw) {
+    return codemap_pack_worst_bytes(n_patches, th, tw);
+}
+
+int vqae_codemap_pack(const void* map, int map_is_u8, int64_t map_rows, int64_t map_cols, int th, int tw,
+                      const uint32_t* freq_host, int num_codes, int scale_bits, int64_t* offsets,
+                      uint8_t* payload, int64_t payload_capacity, void* scratch, size_t scratch_bytes,
+                      void* stream) {
+    return codemap_pack(map, map_is_u8, map_rows, map_cols, th, tw, freq_host, num_codes, scale_bits, offsets,
+                        payload, payload_capacity, scratch, scratch_bytes, (cudaStream_t)stream);
+}
+
+int vqae_codemap_unpack(const uint8_t* payload, int64_t payload_bytes, const int64_t* offsets_host,
+                        const int64_t* offsets, int64_t map_rows, int64_t map_cols, int th, int tw,
+                        const uint32_t* freq_host, int num_codes, int scale_bits, int64_t r0, int64_t c0,
+                        int64_t nr, int64_t nc, void* out, int out_is_u8, uint8_t* flags, void* stream) {
+    return codemap_unpack(payload, payload_bytes, offsets_host, offsets, map_rows, map_cols, th, tw, freq_host,
+                          num_codes, scale_bits, r0, c0, nr, nc, out, out_is_u8, flags, (cudaStream_t)stream);
+}
+
 }  // extern "C"

@@ -182,4 +182,17 @@ int quality_u8(const uint8_t* ref, int64_t ref_rows, int64_t ref_cols, int64_t r
                int W, int64_t* sse, double* ssim, void* scratch, size_t scratch_bytes,
                cudaStream_t stream);
 
+// codemap_pack.cu (packed code maps: histogram, rANS pack, region unpack)
+int codemap_histogram(const void* map, int map_is_u8, int64_t map_rows, int64_t map_cols, int64_t r0,
+                      int64_t c0, int64_t nr, int64_t nc, int K, int64_t* counts, cudaStream_t stream);
+size_t codemap_pack_scratch_bytes(int64_t n_patches, int th, int tw);
+int64_t codemap_pack_worst_bytes(int64_t n_patches, int th, int tw);
+int codemap_pack(const void* map, int map_is_u8, int64_t map_rows, int64_t map_cols, int th, int tw,
+                 const uint32_t* freq_host, int K, int S, int64_t* offsets, uint8_t* payload,
+                 int64_t payload_capacity, void* scratch, size_t scratch_bytes, cudaStream_t stream);
+int codemap_unpack(const uint8_t* payload, int64_t payload_bytes, const int64_t* offsets_host,
+                   const int64_t* offsets, int64_t map_rows, int64_t map_cols, int th, int tw,
+                   const uint32_t* freq_host, int K, int S, int64_t r0, int64_t c0, int64_t nr, int64_t nc,
+                   void* out, int out_is_u8, uint8_t* flags, cudaStream_t stream);
+
 }  // namespace vqae

@@ -10,6 +10,7 @@ import ctypes as C
 import math
 from typing import Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 from . import _lib as L
@@ -996,6 +997,88 @@ def quality_u8(ref_canvas: Tensor, ref_addr: Tuple[int, int, int, int], rec_canv
                                 brc, bfirst, batch, h, w, _ptr(sse), _ptr(ssim), _ptr(ws), ws.numel(),
                                 _stream(dev)), "vqae_quality_u8")
     return sse, ssim
+
+
+def _code_map_arg(code_map: Tensor, what: str) -> Tensor:
+    require_cuda(code_map, what)
+    if code_map.dtype not in (torch.uint8, torch.int64) or code_map.dim() != 2:
+        raise ValueError(f"{what} reads a 2-D uint8 or int64 code map")
+    return code_map.contiguous()
+
+
+def _host_u32(values) -> np.ndarray:
+    return np.ascontiguousarray(np.asarray(values, dtype=np.uint32))
+
+
+def _host_i64(values) -> np.ndarray:
+    if isinstance(values, Tensor):
+        values = values.cpu().numpy()
+    return np.ascontiguousarray(np.asarray(values, dtype=np.int64))
+
+
+def codemap_histogram(code_map: Tensor, k: int, window: Optional[Tuple[int, int, int, int]] = None
+                      ) -> Tuple[Tensor, Tensor]:
+    """Code counts of a uint8 / int64 map, or of the window ``(r0, c0, nr, nc)`` of it in codes
+    (vqae_codemap_histogram): int64 [k] counts of the codes 0 .. k-1 and an int64 scalar counting the
+    codes outside [0, k), both on the map's device."""
+    lib = L.load()
+    code_map = _code_map_arg(code_map, "codemap_histogram")
+    r0, c0, nr, nc = window if window is not None else (0, 0, code_map.shape[0], code_map.shape[1])
+    counts = torch.empty(k + 1, dtype=torch.int64, device=code_map.device)
+    L.check(lib.vqae_codemap_histogram(_ptr(code_map), int(code_map.dtype == torch.uint8), code_map.shape[0],
+                                       code_map.shape[1], r0, c0, nr, nc, k, _ptr(counts),
+                                       _stream(code_map.device)), "vqae_codemap_histogram")
+    return counts[:k], counts[k]
+
+
+def codemap_pack(code_map: Tensor, code_hw: Tuple[int, int], freq, scale_bits: int) -> Tuple[Tensor, Tensor]:
+    """rANS-pack every th x tw patch of a uint8 / int64 map with the frequency table ``freq`` (k entries
+    summing to 2^scale_bits; host values) (vqae_codemap_pack).  Returns the int64 [P + 1] stream offsets
+    and the payload buffer (uint8, worst-case sized: the payload is its first ``offsets[P]`` bytes)."""
+    lib = L.load()
+    code_map = _code_map_arg(code_map, "codemap_pack")
+    th, tw = code_hw
+    fh = _host_u32(freq)
+    dev = code_map.device
+    p = (code_map.shape[0] // th) * (code_map.shape[1] // tw)
+    offsets = torch.empty(p + 1, dtype=torch.int64, device=dev)
+    payload = torch.empty(max(lib.vqae_codemap_pack_worst_bytes(p, th, tw), 1), dtype=torch.uint8, device=dev)
+    ws = workspace(dev, lib.vqae_codemap_pack_scratch_bytes(p, th, tw))
+    L.check(lib.vqae_codemap_pack(_ptr(code_map), int(code_map.dtype == torch.uint8), code_map.shape[0],
+                                  code_map.shape[1], th, tw, fh.ctypes.data_as(C.c_void_p), len(fh), scale_bits,
+                                  _ptr(offsets), _ptr(payload), payload.numel(), _ptr(ws), ws.numel(),
+                                  _stream(dev)), "vqae_codemap_pack")
+    return offsets, payload
+
+
+def codemap_unpack(payload: Tensor, offsets: Tensor, offsets_host, map_hw: Tuple[int, int],
+                   code_hw: Tuple[int, int], freq, scale_bits: int, region: Tuple[int, int, int, int],
+                   dtype: torch.dtype = torch.uint8) -> Tuple[Tensor, Tensor]:
+    """Decode the patches ``region = (r0, c0, nr, nc)`` of a packed map (vqae_codemap_unpack): payload
+    uint8 and offsets int64 [P + 1] on the device, ``offsets_host`` the same offsets on the host, ``freq``
+    the host frequency table.  Returns the [nr*th, nc*tw] map (``dtype`` uint8 or int64) and the uint8
+    [nr, nc] integrity flags (0: the patch decoded back to the encoder's initial state with its words
+    exactly consumed)."""
+    lib = L.load()
+    require_cuda(payload, "codemap_unpack")
+    if payload.dtype != torch.uint8 or offsets.dtype != torch.int64 or offsets.device != payload.device:
+        raise ValueError("codemap_unpack reads a uint8 payload and int64 offsets on one device")
+    if dtype not in (torch.uint8, torch.int64):
+        raise ValueError("codemap_unpack writes uint8 or int64 maps")
+    th, tw = code_hw
+    r0, c0, nr, nc = region
+    fh, oh = _host_u32(freq), _host_i64(offsets_host)
+    if oh.shape != (offsets.numel(),) or offsets.numel() != (map_hw[0] // th) * (map_hw[1] // tw) + 1:
+        raise ValueError("codemap_unpack: offsets do not match the patch grid")
+    dev = payload.device
+    out = torch.empty(nr * th, nc * tw, dtype=dtype, device=dev)
+    flags = torch.empty(nr, nc, dtype=torch.uint8, device=dev)
+    L.check(lib.vqae_codemap_unpack(_ptr(payload), payload.numel(), oh.ctypes.data_as(C.c_void_p),
+                                    _ptr(offsets.contiguous()), map_hw[0], map_hw[1], th, tw,
+                                    fh.ctypes.data_as(C.c_void_p), len(fh), scale_bits, r0, c0, nr, nc,
+                                    _ptr(out), int(dtype == torch.uint8), _ptr(flags), _stream(dev)),
+            "vqae_codemap_unpack")
+    return out, flags
 
 
 # ---- f-4: training-mode codebook maintenance, level sums -------------------------------------------

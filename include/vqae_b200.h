@@ -437,6 +437,47 @@ int vqae_quality_u8(const uint8_t* ref, int64_t ref_rows, int64_t ref_cols, int6
                     int64_t batch, int height, int width, int64_t* sse, double* ssim,
                     void* scratch, size_t scratch_bytes, void* stream);
 
+/* ---- packed code maps: per-patch rANS entropy coding (csrc/codemap_pack.cu, DESIGN.md 4.13) ---
+ * A code map [map_rows, map_cols] (uint8 when map_is_u8 / out_is_u8, else int64) is a grid of th x tw
+ * code tiles; patch p = row-major patch index.  Format version 1: one static table of num_codes (K)
+ * frequencies freq_host[s] summing to 2^scale_bits (S), one rANS stream per patch (32-bit state,
+ * L = 2^16, 16-bit words): the final encoder state (4 bytes LE), then the words in decoder order (2 bytes
+ * LE each); 4 <= stream bytes <= 4 + 2 th tw, always even.  offsets [P + 1] (int64): stream p is
+ * payload[offsets[p], offsets[p + 1]), offsets[0] = 0, offsets[P] = payload bytes.
+ *
+ * vqae_codemap_histogram   counts[K + 1] (int64): counts[s] = #codes equal to s in the window
+ *                          rows [r0, r0 + nr) x cols [c0, c0 + nc) of the map (in codes), counts[K] = #codes
+ *                          outside [0, K).  Exact (integer atomics), independent of the grid.
+ * vqae_codemap_pack        codes every patch of the whole map with the table: writes offsets and the
+ *                          payload (payload_capacity >= vqae_codemap_pack_worst_bytes).  A patch holding a
+ *                          code outside [0, K) or with frequency 0 gets a 0-byte stream (offsets show it).
+ * vqae_codemap_unpack      decodes the patches of the region (r0, c0, nr, nc) (in patches) into out
+ *                          [nr th, nc tw] (patch t of the region, row-major, at (t / nc, t % nc) -- the
+ *                          addressing of vqae_codemap_place_u8 with grid_cols = nc) and writes flags[nr nc]:
+ *                          bit 0 the final state is not L, bit 1 the words were not exactly consumed,
+ *                          bit 2 the stream length is not even within [4, 4 + 2 th tw].  offsets_host and
+ *                          offsets hold the same P + 1 values (host copy validated, device copy read).
+ *                          Every read of patch p stays inside its own [offsets[p], offsets[p + 1]) range
+ *                          clamped to the payload; past its end a stream reads zero words.
+ * Checked before anything is launched: VQAE_ERR_BAD_ARG for a null pointer, a non-positive extent, a
+ * map that is not a grid of tiles, a window or region outside the map, frequencies not summing to 2^S,
+ * offsets that do not start at 0, end at payload_bytes and step by an even 4 .. 4 + 2 th tw, or a short
+ * payload_capacity; VQAE_ERR_UNSUPPORTED for K outside [1, 1024], S outside [1, 14], th tw > 16384,
+ * more than 2^31 - 1 patches, or a uint8 output with K > 256; VQAE_ERR_SCRATCH when scratch is missing
+ * or smaller than vqae_codemap_pack_scratch_bytes.                                                 */
+int vqae_codemap_histogram(const void* map, int map_is_u8, int64_t map_rows, int64_t map_cols, int64_t r0,
+                           int64_t c0, int64_t nr, int64_t nc, int num_codes, int64_t* counts, void* stream);
+size_t vqae_codemap_pack_scratch_bytes(int64_t n_patches, int th, int tw);
+int64_t vqae_codemap_pack_worst_bytes(int64_t n_patches, int th, int tw);
+int vqae_codemap_pack(const void* map, int map_is_u8, int64_t map_rows, int64_t map_cols, int th, int tw,
+                      const uint32_t* freq_host, int num_codes, int scale_bits, int64_t* offsets,
+                      uint8_t* payload, int64_t payload_capacity, void* scratch, size_t scratch_bytes,
+                      void* stream);
+int vqae_codemap_unpack(const uint8_t* payload, int64_t payload_bytes, const int64_t* offsets_host,
+                        const int64_t* offsets, int64_t map_rows, int64_t map_cols, int th, int tw,
+                        const uint32_t* freq_host, int num_codes, int scale_bits, int64_t r0, int64_t c0,
+                        int64_t nr, int64_t nc, void* out, int out_is_u8, uint8_t* flags, void* stream);
+
 /* ---- f-4  training-mode codebook maintenance (layers/vq.py:47-94) -----------------------------
  * EMAVectorQuantizer._update_ema / _init_ema without the N x K one-hot matrix of the reference:
  *   vqae_ema_accumulate_f32   counts[k] = #{n : idx[n] = k},  dw[k,:] = sum of z[n,:] over those n
