@@ -582,4 +582,18 @@ int vqae_codemap_unpack(const uint8_t* payload, int64_t payload_bytes, const int
                           num_codes, scale_bits, r0, c0, nr, nc, out, out_is_u8, flags, (cudaStream_t)stream);
 }
 
+size_t vqae_pyramid_u8_scratch_bytes(int64_t batch, int height, int width, int level_mask) {
+    return pyramid_u8_scratch_bytes(batch, height, width, level_mask);
+}
+
+int vqae_pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int64_t src_r0, int64_t src_c0,
+                    int64_t src_region_cols, int64_t src_first, int64_t batch, int height, int width,
+                    int level_mask, uint8_t* const* dst, const int64_t* dst_rows, const int64_t* dst_cols,
+                    int64_t dst_r0, int64_t dst_c0, int64_t dst_region_cols, int64_t dst_first,
+                    void* scratch, size_t scratch_bytes, void* stream) {
+    return pyramid_u8(src, src_rows, src_cols, src_r0, src_c0, src_region_cols, src_first, batch, height, width,
+                      level_mask, dst, dst_rows, dst_cols, dst_r0, dst_c0, dst_region_cols, dst_first, scratch,
+                      scratch_bytes, (cudaStream_t)stream);
+}
+
 }  // extern "C"

@@ -195,4 +195,12 @@ int codemap_unpack(const uint8_t* payload, int64_t payload_bytes, const int64_t*
                    const uint32_t* freq_host, int K, int S, int64_t r0, int64_t c0, int64_t nr, int64_t nc,
                    void* out, int out_is_u8, uint8_t* flags, cudaStream_t stream);
 
+// pyramid.cu (box-filtered levels 2^1 .. 2^9 of uint8 RGB patches)
+size_t pyramid_u8_scratch_bytes(int64_t batch, int H, int W, int mask);
+int pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int64_t src_r0, int64_t src_c0,
+               int64_t src_rc, int64_t src_first, int64_t batch, int H, int W, int mask,
+               uint8_t* const* dst, const int64_t* dst_rows, const int64_t* dst_cols, int64_t dst_r0,
+               int64_t dst_c0, int64_t dst_rc, int64_t dst_first, void* scratch, size_t scratch_bytes,
+               cudaStream_t stream);
+
 }  // namespace vqae

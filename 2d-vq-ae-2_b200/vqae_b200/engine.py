@@ -999,6 +999,36 @@ def quality_u8(ref_canvas: Tensor, ref_addr: Tuple[int, int, int, int], rec_canv
     return sse, ssim
 
 
+def pyramid_u8(src_canvas: Tensor, src_addr: Tuple[int, int, int, int], batch: int, h: int, w: int,
+               dst: Dict[int, Tensor], dst_addr: Tuple[int, int, int, int]) -> None:
+    """Box-filtered levels of ``batch`` h x w patches of a uint8 RGB canvas (vqae_pyramid_u8): for every
+    factor f of ``dst`` (a power of two in [2, 512] dividing h and w), ``dst[f]`` receives per channel
+    (S + f^2 / 2) >> log2(f^2), S the exact sum of each f x f block -- ``PIL.Image.reduce(f)``.  Every
+    canvas is a contiguous uint8 [rows, cols, 3] tensor; ``addr = (r0, c0, region_cols, first)`` puts
+    patch t at grid position (r0 + (first + t) // region_cols, c0 + (first + t) % region_cols), of h x w
+    patches in the source and of h/f x w/f patches in ``dst[f]``."""
+    from .pyramid import check_factors
+    lib = L.load()
+    require_cuda(src_canvas, "pyramid_u8")
+    factors = check_factors(dst.keys(), (h, w))
+    for cv in (src_canvas, *dst.values()):
+        if cv.dtype != torch.uint8 or cv.dim() != 3 or cv.shape[2] != 3 or not cv.is_contiguous() or \
+                cv.device != src_canvas.device:
+            raise ValueError("pyramid_u8 reads and writes contiguous uint8 [rows, cols, 3] canvases on one device")
+    ptrs, rows, cols = (C.c_void_p * 10)(), (C.c_int64 * 10)(), (C.c_int64 * 10)()
+    mask = 0
+    for f in factors:
+        k = f.bit_length() - 1
+        mask |= 1 << k
+        ptrs[k], rows[k], cols[k] = dst[f].data_ptr(), dst[f].shape[0], dst[f].shape[1]
+    dev = src_canvas.device
+    ws = workspace(dev, lib.vqae_pyramid_u8_scratch_bytes(batch, h, w, mask))
+    (sr0, sc0, src_rc, sfirst), (dr0, dc0, drc, dfirst) = src_addr, dst_addr
+    L.check(lib.vqae_pyramid_u8(_ptr(src_canvas), src_canvas.shape[0], src_canvas.shape[1], sr0, sc0, src_rc,
+                                sfirst, batch, h, w, mask, ptrs, rows, cols, dr0, dc0, drc, dfirst, _ptr(ws),
+                                ws.numel(), _stream(dev)), "vqae_pyramid_u8")
+
+
 def _code_map_arg(code_map: Tensor, what: str) -> Tensor:
     require_cuda(code_map, what)
     if code_map.dtype not in (torch.uint8, torch.int64) or code_map.dim() != 2:

@@ -21,6 +21,7 @@ from . import engine as E
 from . import plan as P
 from .graphs import CapturedStep
 from .plan import resolve_precision
+from .pyramid import check_factors, level_canvases
 from .quality import ReconstructionQuality, check_u8_patches, reconstruction_quality
 from .sharding import gather_code_tiles, shard_range, slide_grid  # noqa: F401
 
@@ -375,6 +376,31 @@ def score_region(model, code_map: torch.Tensor, code_hw: Tuple[int, int], slide_
         sse[first:first + n], ssim[first:first + n] = E.quality_u8(slide_u8, (r0, c0, nc, first), rec,
                                                                    (0, 0, 1, 0), n, h, w)
     return ReconstructionQuality(sse.view(nr, nc, 3), ssim.view(nr, nc), (h, w))
+
+
+@torch.no_grad()
+def decompress_pyramid(model, code_map: torch.Tensor, code_hw: Tuple[int, int], factors: Iterable[int],
+                       region: Optional[Tuple[int, int, int, int]] = None, batch: int = 256, mean=None,
+                       std=None) -> Dict[int, torch.Tensor]:
+    """The pyramid levels of a decoded code map without its full-resolution canvas: decode the region
+    (as ``decompress_region`` does, at most ``batch`` patches per step into one reused buffer) and reduce
+    each decoded batch to every level right away.  Returns ``{f: uint8 [nr*H/f, nc*W/f, 3]}`` for the
+    region ``(r0, c0, nr, nc)`` (default the whole map), equal byte for byte to ``slide_pyramid`` of
+    ``decompress_region``'s output; ``factors`` as in ``pyramid.check_factors``.  Argument checks as in
+    ``decompress_region``.  A packed map goes through ``packing.unpack_code_map`` first."""
+    pq, dec, code_map, (th, tw), _, (r0, c0, nr, nc), f = _region_plan(model, code_map, code_hw, region,
+                                                                       batch, "decompress_pyramid")
+    h, w = th * f, tw * f
+    levels = level_canvases((nr, nc), (h, w), check_factors(factors, (h, w)), code_map.device)
+    total = nr * nc
+    buf = torch.empty(min(batch, total) * h, w, 3, dtype=torch.uint8, device=code_map.device)
+    for first in range(0, total, batch):
+        n = min(batch, total - first)
+        enc = E.embed_codemap(pq, code_map, (th, tw), r0, c0, nc, first, n)
+        rec = buf[:n * h]
+        P.decoder_forward_u8(dec, enc, mean, std, rec, 0, 1)
+        E.pyramid_u8(rec, (0, 0, 1, 0), n, h, w, levels, (0, 0, nc, first))
+    return levels
 
 
 def tiles_to_map(tiles_u8: torch.Tensor, grid: Tuple[int, int]) -> torch.Tensor:

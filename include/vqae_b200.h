@@ -478,6 +478,29 @@ int vqae_codemap_unpack(const uint8_t* payload, int64_t payload_bytes, const int
                         const uint32_t* freq_host, int num_codes, int scale_bits, int64_t r0, int64_t c0,
                         int64_t nr, int64_t nc, void* out, int out_is_u8, uint8_t* flags, void* stream);
 
+/* ---- box-filtered pyramid levels of uint8 RGB patches (csrc/pyramid.cu, DESIGN.md 4.14) ----------
+ * Level k of the bit mask level_mask (bit k: factor f = 2^k, 1 <= k <= 9, f dividing height and width)
+ * is, per channel, out = (S + f^2 / 2) >> 2k with S the exact integer sum of the f x f source pixels:
+ * the box mean rounded half up (PIL.Image.reduce(f)), every level rounded once from the original
+ * pixels.  The source is a canvas uint8 [src_rows, src_cols, 3] of height x width patches; patch t of the
+ * call sits at grid position (r0 + (first + t) / region_cols, c0 + (first + t) % region_cols) -- the
+ * addressing of vqae_quality_u8.  Level k goes to the canvas dst[k] uint8 [dst_rows[k], dst_cols[k], 3]
+ * of (height / f) x (width / f) patches, at the position the dst_* tuple (shared by all levels) gives
+ * patch t.  dst, dst_rows and dst_cols are host arrays of 10 entries indexed by k; entries of levels
+ * not in the mask are not read.  Each source pixel is read once; integer arithmetic, no atomics: bitwise
+ * reproducible, independent of the batch and the grid.  Checked before anything is launched:
+ * VQAE_ERR_BAD_ARG for a null pointer (src, the arrays, dst[k] of a requested level), a non-positive
+ * extent, an empty mask, a negative first or a placement outside any canvas; VQAE_ERR_UNSUPPORTED for
+ * mask bits outside 1 .. 9, a factor not dividing height or width, or first + batch > 2^31;
+ * VQAE_ERR_SCRATCH when vqae_pyramid_u8_scratch_bytes is nonzero (levels with f >= 128) and scratch is
+ * missing or smaller (0 for an unsupported shape).                                                   */
+size_t vqae_pyramid_u8_scratch_bytes(int64_t batch, int height, int width, int level_mask);
+int vqae_pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int64_t src_r0, int64_t src_c0,
+                    int64_t src_region_cols, int64_t src_first, int64_t batch, int height, int width,
+                    int level_mask, uint8_t* const* dst, const int64_t* dst_rows, const int64_t* dst_cols,
+                    int64_t dst_r0, int64_t dst_c0, int64_t dst_region_cols, int64_t dst_first,
+                    void* scratch, size_t scratch_bytes, void* stream);
+
 /* ---- f-4  training-mode codebook maintenance (layers/vq.py:47-94) -----------------------------
  * EMAVectorQuantizer._update_ema / _init_ema without the N x K one-hot matrix of the reference:
  *   vqae_ema_accumulate_f32   counts[k] = #{n : idx[n] = k},  dw[k,:] = sum of z[n,:] over those n
