@@ -118,6 +118,14 @@ SIGNATURES = {
     "vqae_codemap_pack": (_i, [_vp, _i, _i64, _i64, _i, _i, _vp, _i, _i, _vp, _vp, _i64, _vp, _sz, _vp]),
     "vqae_codemap_unpack": (_i, [_vp, _i64, _vp, _vp, _i64, _i64, _i, _i, _vp, _i, _i, _i64, _i64, _i64, _i64,
                                  _vp, _i, _vp, _vp]),
+    "vqae_residual_stats": (_i, [_vp, _i64, _i64, _i64, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _i64, _i64,
+                                 _i64, _i, _i, _i, _vp, _vp, _vp]),
+    "vqae_residual_tables": (_i, [_vp, _i64, _vp, _vp]),
+    "vqae_residual_encode_scratch_bytes": (_sz, [_i64, _i, _i]),
+    "vqae_residual_encode": (_i, [_vp, _i64, _i64, _i64, _i64, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _i64, _i64,
+                                  _i64, _i, _i, _i, _vp, _vp, _vp, _i64, _vp, _sz, _vp]),
+    "vqae_residual_apply": (_i, [_vp, _i64, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _i64, _i64, _vp, _i64, _i64,
+                                 _i64, _i64, _i64, _i64, _i64, _i, _i, _i, _vp, _vp]),
     "vqae_pyramid_u8_scratch_bytes": (_sz, [_i64, _i, _i, _i]),
     "vqae_pyramid_u8": (_i, [_vp, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i, _i, _i, _vp, _vp, _vp, _i64, _i64,
                              _i64, _i64, _vp, _sz, _vp]),

@@ -596,4 +596,44 @@ int vqae_pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int6
                       scratch_bytes, (cudaStream_t)stream);
 }
 
+int vqae_residual_stats(const uint8_t* x, int64_t x_rows, int64_t x_cols, int64_t x_r0, int64_t x_c0,
+                        int64_t x_region_cols, int64_t x_first, const uint8_t* base, int64_t base_rows,
+                        int64_t base_cols, int64_t base_r0, int64_t base_c0, int64_t base_region_cols,
+                        int64_t base_first, int64_t batch, int height, int width, int max_error, int64_t* hist,
+                        uint32_t* adler, void* stream) {
+    return residual_stats(x, x_rows, x_cols, x_r0, x_c0, x_region_cols, x_first, base, base_rows, base_cols,
+                          base_r0, base_c0, base_region_cols, base_first, batch, height, width, max_error, hist,
+                          adler, (cudaStream_t)stream);
+}
+
+int vqae_residual_tables(const int64_t* hist, int64_t batch, int32_t* freq, void* stream) {
+    return residual_tables(hist, batch, freq, (cudaStream_t)stream);
+}
+
+size_t vqae_residual_encode_scratch_bytes(int64_t batch, int height, int width) {
+    return residual_encode_scratch_bytes(batch, height, width);
+}
+
+int vqae_residual_encode(const uint8_t* x, int64_t x_rows, int64_t x_cols, int64_t x_r0, int64_t x_c0,
+                         int64_t x_region_cols, int64_t x_first, const uint8_t* base, int64_t base_rows,
+                         int64_t base_cols, int64_t base_r0, int64_t base_c0, int64_t base_region_cols,
+                         int64_t base_first, int64_t batch, int height, int width, int max_error,
+                         const int32_t* freq, int64_t* offsets, uint8_t* payload, int64_t payload_capacity,
+                         void* scratch, size_t scratch_bytes, void* stream) {
+    return residual_encode(x, x_rows, x_cols, x_r0, x_c0, x_region_cols, x_first, base, base_rows, base_cols,
+                           base_r0, base_c0, base_region_cols, base_first, batch, height, width, max_error, freq,
+                           offsets, payload, payload_capacity, scratch, scratch_bytes, (cudaStream_t)stream);
+}
+
+int vqae_residual_apply(const uint8_t* payload, int64_t payload_bytes, const int64_t* offsets_host,
+                        const int64_t* offsets, const uint32_t* adler, int64_t grid_rows, int64_t grid_cols,
+                        int64_t layer_r0, int64_t layer_c0, int64_t layer_region_cols, int64_t layer_first,
+                        uint8_t* canvas, int64_t rows, int64_t cols, int64_t r0, int64_t c0, int64_t region_cols,
+                        int64_t first, int64_t batch, int height, int width, int max_error, uint8_t* flags,
+                        void* stream) {
+    return residual_apply(payload, payload_bytes, offsets_host, offsets, adler, grid_rows, grid_cols, layer_r0,
+                          layer_c0, layer_region_cols, layer_first, canvas, rows, cols, r0, c0, region_cols, first,
+                          batch, height, width, max_error, flags, (cudaStream_t)stream);
+}
+
 }  // extern "C"

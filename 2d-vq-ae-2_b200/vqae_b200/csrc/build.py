@@ -22,11 +22,11 @@ STAMP = PKG / ".libvqae_b200.stamp"
 SOURCES = ["abi.cu", "conv_f32.cu", "stems.cu", "quantize.cu", "quantize_tc.cu", "tc_kernels.cu",
            "tc_down.cu", "tc_chain.cu", "tc_resident.cu", "up_tail.cu", "up_head.cu", "pack.cu",
            "mma_same.cu", "mma_down.cu", "mma_up.cu", "tc_split.cu", "mma_front.cu", "mma_stem.cu", "tc_down128.cu", "mma_same_split.cu", "ema.cu", "mbconv.cu",
-           "quality.cu", "codemap_pack.cu", "pyramid.cu"]
+           "quality.cu", "codemap_pack.cu", "pyramid.cu", "residual.cu"]
 # test / measurement aids: a separate library that links against the product library
 AID_SOURCES = ["testaids.cu", "tc_bench.cu"]
 AIDS_PATH = PKG / "libvqae_b200_testaids.so"
-HEADERS = ["common.cuh", "kernels.cuh", "tc_common.cuh", "mma_common.cuh"]
+HEADERS = ["common.cuh", "kernels.cuh", "tc_common.cuh", "mma_common.cuh", "rans.cuh"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -31,12 +31,13 @@
 // the payload, the tables or the patch's own buffer.
 #include "common.cuh"
 #include "kernels.cuh"
+#include "rans.cuh"
 
 namespace vqae {
 
 namespace {
 
-constexpr uint32_t PK_L = 1u << 16;           // lower end of the state interval
+constexpr uint32_t PK_L = RANS_L;
 constexpr int PK_MAX_K = 1024;                // the quantiser's own codebook limit
 constexpr int PK_MAX_S = 14;
 constexpr int PK_MAX_CODES = 16384;           // th * tw
@@ -130,12 +131,11 @@ codemap_encode_kernel(const MapT* __restrict__ map, int64_t map_cols, int64_t gr
                 f = 1u << S;
                 c = 0;
             }
-            if ((uint64_t)x >= ((uint64_t)f << (32 - S))) {
-                t[n - 1 - w] = (uint16_t)(x & 0xffffu);     // position >= i: already read
+            uint16_t word;
+            if (rans_encode(x, f, c, S, word)) {
+                t[n - 1 - w] = word;                        // position >= i: already read
                 ++w;
-                x >>= 16;
             }
-            x = ((x / f) << S) + x % f + c;
         }
         st_state[tid] = x;
         st_words[tid] = w;
@@ -399,9 +399,14 @@ int codemap_pack(const void* map, int map_is_u8, int64_t map_rows, int64_t map_c
             static_cast<const int64_t*>(map), map_cols, gc, P, th, tw, stride, ppc, K, S, tab, slots, sb, sizes);
     }
     if (int rc = check_launch()) return rc;
+    return rans_offsets_and_compact(sizes, P, slots, sb, offsets, payload, payload_capacity, stream);
+}
+
+int rans_offsets_and_compact(const uint32_t* sizes, int64_t P, const uint8_t* slots, int64_t slot_bytes,
+                             int64_t* offsets, uint8_t* payload, int64_t capacity, cudaStream_t stream) {
     codemap_offsets_kernel<<<1, PK_SCAN_THREADS, 0, stream>>>(sizes, P, offsets);
     if (int rc = check_launch()) return rc;
-    codemap_compact_kernel<<<ceil_div_u(P, 8), 256, 0, stream>>>(slots, sb, offsets, P, payload, payload_capacity);
+    codemap_compact_kernel<<<ceil_div_u(P, 8), 256, 0, stream>>>(slots, slot_bytes, offsets, P, payload, capacity);
     return check_launch();
 }
 

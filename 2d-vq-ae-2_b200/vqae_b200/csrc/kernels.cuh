@@ -195,6 +195,24 @@ int codemap_unpack(const uint8_t* payload, int64_t payload_bytes, const int64_t*
                    const uint32_t* freq_host, int K, int S, int64_t r0, int64_t c0, int64_t nr, int64_t nc,
                    void* out, int out_is_u8, uint8_t* flags, cudaStream_t stream);
 
+// residual.cu (near-lossless residual layer of stored code maps: stats, tables, encode, apply)
+int residual_stats(const uint8_t* x, int64_t x_rows, int64_t x_cols, int64_t x_r0, int64_t x_c0, int64_t x_rc,
+                   int64_t x_first, const uint8_t* base, int64_t b_rows, int64_t b_cols, int64_t b_r0, int64_t b_c0,
+                   int64_t b_rc, int64_t b_first, int64_t batch, int H, int W, int e, int64_t* hist,
+                   uint32_t* adler, cudaStream_t stream);
+int residual_tables(const int64_t* hist, int64_t batch, int32_t* freq, cudaStream_t stream);
+size_t residual_encode_scratch_bytes(int64_t batch, int H, int W);
+int residual_encode(const uint8_t* x, int64_t x_rows, int64_t x_cols, int64_t x_r0, int64_t x_c0, int64_t x_rc,
+                    int64_t x_first, const uint8_t* base, int64_t b_rows, int64_t b_cols, int64_t b_r0,
+                    int64_t b_c0, int64_t b_rc, int64_t b_first, int64_t batch, int H, int W, int e,
+                    const int32_t* freq, int64_t* offsets, uint8_t* payload, int64_t payload_capacity,
+                    void* scratch, size_t scratch_bytes, cudaStream_t stream);
+int residual_apply(const uint8_t* payload, int64_t payload_bytes, const int64_t* offsets_host,
+                   const int64_t* offsets, const uint32_t* adler, int64_t grid_rows, int64_t grid_cols,
+                   int64_t l_r0, int64_t l_c0, int64_t l_rc, int64_t l_first, uint8_t* canvas, int64_t rows,
+                   int64_t cols, int64_t r0, int64_t c0, int64_t rc, int64_t first, int64_t batch, int H, int W,
+                   int e, uint8_t* flags, cudaStream_t stream);
+
 // pyramid.cu (box-filtered levels 2^1 .. 2^9 of uint8 RGB patches)
 size_t pyramid_u8_scratch_bytes(int64_t batch, int H, int W, int mask);
 int pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int64_t src_r0, int64_t src_c0,

@@ -1029,6 +1029,96 @@ def pyramid_u8(src_canvas: Tensor, src_addr: Tuple[int, int, int, int], batch: i
                                 ws.numel(), _stream(dev)), "vqae_pyramid_u8")
 
 
+RESIDUAL_HEADER_BYTES = 768        # 256 x u16 frequencies, 32 x u32 word counts, 32 x u32 final states
+
+
+def _canvas_args(canvas: Tensor, addr: Tuple[int, int, int, int], what: str, device) -> list:
+    if canvas.dtype != torch.uint8 or canvas.dim() != 3 or canvas.shape[2] != 3 or not canvas.is_contiguous() \
+            or canvas.device != device:
+        raise ValueError(f"{what} reads contiguous uint8 [rows, cols, 3] canvases on one device")
+    r0, c0, rc, first = addr
+    return [_ptr(canvas), canvas.shape[0], canvas.shape[1], r0, c0, rc, first]
+
+
+def residual_stats(x_canvas: Tensor, x_addr: Tuple[int, int, int, int], base_canvas: Tensor,
+                   base_addr: Tuple[int, int, int, int], batch: int, h: int, w: int, max_error: int
+                   ) -> Tuple[Tensor, Tensor]:
+    """Residual symbol histograms (int64 [batch, 256]) and Adler-32 values (int32 [batch, 2]: of the base
+    pixels and of the reconstruction x', the uint32 bits) of ``batch`` h x w patches (vqae_residual_stats);
+    canvases and ``addr`` tuples as in ``quality_u8``."""
+    lib = L.load()
+    require_cuda(x_canvas, "residual_stats")
+    dev = x_canvas.device
+    hist = torch.empty(batch, 256, dtype=torch.int64, device=dev)
+    adler = torch.empty(batch, 2, dtype=torch.int32, device=dev)
+    L.check(lib.vqae_residual_stats(*_canvas_args(x_canvas, x_addr, "residual_stats", dev),
+                                    *_canvas_args(base_canvas, base_addr, "residual_stats", dev), batch, h, w,
+                                    max_error, _ptr(hist), _ptr(adler), _stream(dev)), "vqae_residual_stats")
+    return hist, adler
+
+
+def residual_tables(hist: Tensor) -> Tensor:
+    """Per-patch rANS tables int32 [batch, 256] (total 2^14) of int64 [batch, 256] symbol counts: the rule of
+    ``packing.quantise_frequencies`` on the GPU (vqae_residual_tables)."""
+    lib = L.load()
+    require_cuda(hist, "residual_tables")
+    if hist.dtype != torch.int64 or hist.dim() != 2 or hist.shape[1] != 256 or not hist.is_contiguous():
+        raise ValueError("residual_tables reads contiguous int64 [batch, 256] counts")
+    freq = torch.empty(hist.shape, dtype=torch.int32, device=hist.device)
+    L.check(lib.vqae_residual_tables(_ptr(hist), hist.shape[0], _ptr(freq), _stream(hist.device)),
+            "vqae_residual_tables")
+    return freq
+
+
+def residual_encode(x_canvas: Tensor, x_addr: Tuple[int, int, int, int], base_canvas: Tensor,
+                    base_addr: Tuple[int, int, int, int], batch: int, h: int, w: int, max_error: int,
+                    freq: Tensor) -> Tuple[Tensor, Tensor]:
+    """Residual chunks of ``batch`` patches coded with their tables ``freq`` (int32 [batch, 256], from
+    ``residual_tables``) (vqae_residual_encode).  Returns the int64 [batch + 1] chunk offsets and the payload
+    buffer (uint8, worst-case sized: the payload is its first ``offsets[batch]`` bytes)."""
+    lib = L.load()
+    require_cuda(x_canvas, "residual_encode")
+    dev = x_canvas.device
+    if freq.dtype != torch.int32 or tuple(freq.shape) != (batch, 256) or not freq.is_contiguous() \
+            or freq.device != dev:
+        raise ValueError(f"residual_encode reads contiguous int32 [{batch}, 256] tables on {dev}")
+    offsets = torch.empty(batch + 1, dtype=torch.int64, device=dev)
+    payload = torch.empty(batch * (RESIDUAL_HEADER_BYTES + 6 * h * w), dtype=torch.uint8, device=dev)
+    ws = workspace(dev, lib.vqae_residual_encode_scratch_bytes(batch, h, w))
+    L.check(lib.vqae_residual_encode(*_canvas_args(x_canvas, x_addr, "residual_encode", dev),
+                                     *_canvas_args(base_canvas, base_addr, "residual_encode", dev), batch, h, w,
+                                     max_error, _ptr(freq), _ptr(offsets), _ptr(payload), payload.numel(),
+                                     _ptr(ws), ws.numel(), _stream(dev)), "vqae_residual_encode")
+    return offsets, payload
+
+
+def residual_apply(payload: Tensor, offsets: Tensor, offsets_host, adler: Tensor, grid: Tuple[int, int],
+                   layer_addr: Tuple[int, int, int, int], canvas: Tensor, addr: Tuple[int, int, int, int],
+                   batch: int, h: int, w: int, max_error: int, flags: Tensor) -> None:
+    """Replace the base pixels of ``batch`` h x w patches of ``canvas`` (placed by ``addr``) by the residual
+    layer's reconstruction, in place (vqae_residual_apply).  Patch t reads the chunk of layer patch
+    (r0 + q // rc, c0 + q % rc), q = first + t, for ``layer_addr = (r0, c0, rc, first)`` in the ``grid`` =
+    (rows, cols) of the layer; ``offsets`` int64 [P + 1] (and the same values on the host), ``adler`` int32
+    [P, 2].  ``flags`` uint8 [batch] receives bit 0 stream, bit 1 base mismatch, bit 2 output mismatch."""
+    lib = L.load()
+    require_cuda(payload, "residual_apply")
+    dev = payload.device
+    if payload.dtype != torch.uint8 or offsets.dtype != torch.int64 or adler.dtype != torch.int32 or \
+            flags.dtype != torch.uint8 or any(t.device != dev or not t.is_contiguous()
+                                              for t in (offsets, adler, flags)):
+        raise ValueError("residual_apply reads a uint8 payload, int64 offsets, int32 Adler values and writes "
+                         "uint8 flags, contiguous on one device")
+    oh = _host_i64(offsets_host)
+    p = grid[0] * grid[1]
+    if oh.shape != (p + 1,) or offsets.numel() != p + 1 or tuple(adler.shape) != (p, 2) or flags.numel() < batch:
+        raise ValueError("residual_apply: offsets / Adler values do not match the patch grid")
+    lr0, lc0, lrc, lfirst = layer_addr
+    L.check(lib.vqae_residual_apply(_ptr(payload), payload.numel(), oh.ctypes.data_as(C.c_void_p), _ptr(offsets),
+                                    _ptr(adler), grid[0], grid[1], lr0, lc0, lrc, lfirst,
+                                    *_canvas_args(canvas, addr, "residual_apply", dev), batch, h, w, max_error,
+                                    _ptr(flags), _stream(dev)), "vqae_residual_apply")
+
+
 def _code_map_arg(code_map: Tensor, what: str) -> Tensor:
     require_cuda(code_map, what)
     if code_map.dtype not in (torch.uint8, torch.int64) or code_map.dim() != 2:

@@ -23,6 +23,7 @@ from .graphs import CapturedStep
 from .plan import resolve_precision
 from .pyramid import check_factors, level_canvases
 from .quality import ReconstructionQuality, check_u8_patches, reconstruction_quality
+from .residual import ResidualIntegrityError, ResidualLayer, check_max_error, check_offsets, flag_causes
 from .sharding import gather_code_tiles, shard_range, slide_grid  # noqa: F401
 
 
@@ -401,6 +402,98 @@ def decompress_pyramid(model, code_map: torch.Tensor, code_hw: Tuple[int, int], 
         P.decoder_forward_u8(dec, enc, mean, std, rec, 0, 1)
         E.pyramid_u8(rec, (0, 0, 1, 0), n, h, w, levels, (0, 0, nc, first))
     return levels
+
+
+@torch.no_grad()
+def encode_residual(model, code_map: torch.Tensor, code_hw: Tuple[int, int], slide_u8: torch.Tensor,
+                    max_error: int = 0, batch: int = 256, mean=None, std=None) -> ResidualLayer:
+    """The near-lossless residual layer of a stored code map against the slide it was made from: decode the
+    map (as ``decompress_region`` does, at most ``batch`` patches per step into one reused buffer) and code
+    each decoded batch's difference to the slide, in place, so that ``decompress_region_exact`` returns every
+    byte within ``max_error`` of ``slide_u8`` (exactly ``slide_u8`` for 0).  ``slide_u8``: contiguous uint8
+    [rows*H, cols*W, 3] on the map's device.  The layer records ``resolve_precision(model.decoder)``: its
+    base pixels are those of that mode.  Argument checks as in ``decompress_region``; a packed map goes
+    through ``packing.unpack_code_map`` first."""
+    e = check_max_error(max_error)
+    pq, dec, code_map, (th, tw), (rows, cols), _, f = _region_plan(model, code_map, code_hw, None, batch,
+                                                                  "encode_residual")
+    h, w = th * f, tw * f
+    shape = (rows * h, cols * w, 3)
+    if not isinstance(slide_u8, torch.Tensor) or tuple(slide_u8.shape) != shape or \
+            slide_u8.dtype != torch.uint8 or slide_u8.device != code_map.device or not slide_u8.is_contiguous():
+        raise ValueError(f"slide_u8 must be a contiguous uint8 tensor of shape {shape} on {code_map.device}")
+    precision = resolve_precision(dec)
+    total = rows * cols
+    adler = torch.empty(total, 2, dtype=torch.int32, device=code_map.device)
+    buf = torch.empty(min(batch, total) * h, w, 3, dtype=torch.uint8, device=code_map.device)
+    chunks, sizes = [], [np.zeros(1, np.int64)]
+    for first in range(0, total, batch):
+        n = min(batch, total - first)
+        enc = E.embed_codemap(pq, code_map, (th, tw), 0, 0, cols, first, n)
+        rec = buf[:n * h]
+        P.decoder_forward_u8(dec, enc, mean, std, rec, 0, 1)
+        hist, adler[first:first + n] = E.residual_stats(slide_u8, (0, 0, cols, first), rec, (0, 0, 1, 0), n, h,
+                                                        w, e)
+        off, payload = E.residual_encode(slide_u8, (0, 0, cols, first), rec, (0, 0, 1, 0), n, h, w, e,
+                                         E.residual_tables(hist))
+        off = off.cpu().numpy()
+        check_offsets(off, 3 * h * w)
+        chunks.append(payload[:int(off[-1])].clone())
+        sizes.append(np.diff(off))
+    offsets = np.cumsum(np.concatenate(sizes)).astype(np.int64)
+    return ResidualLayer(payload=torch.cat(chunks), offsets=torch.from_numpy(offsets).to(code_map.device),
+                         adler=adler, max_error=e, precision=precision, grid=(rows, cols), patch_hw=(h, w),
+                         offsets_host=offsets)
+
+
+@torch.no_grad()
+def decompress_region_exact(model, code_map: torch.Tensor, code_hw: Tuple[int, int], residual: ResidualLayer,
+                            region: Optional[Tuple[int, int, int, int]] = None, batch: int = 256, mean=None,
+                            std=None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """``decompress_region`` followed by the residual layer: every byte of the result is within
+    ``residual.max_error`` of the original slide (equal to it for 0).  Each batch is decoded into the result
+    (``out`` if given) and its residual applied there in place.  Raises ValueError before any launch when the
+    decoder's precision mode is not the one the layer was made with, or the map's grid or patch size is not
+    the layer's; raises ``ResidualIntegrityError`` (a ValueError) naming the patches that failed their checks
+    and the cause of each.  Other arguments as in ``decompress_region``."""
+    pq, dec, code_map, (th, tw), (rows, cols), (r0, c0, nr, nc), f = _region_plan(
+        model, code_map, code_hw, region, batch, "decompress_region_exact")
+    h, w = th * f, tw * f
+    if tuple(residual.grid) != (rows, cols) or tuple(residual.patch_hw) != (h, w):
+        raise ValueError(f"the residual layer covers {residual.grid[0]} x {residual.grid[1]} patches of "
+                         f"{residual.patch_hw[0]} x {residual.patch_hw[1]} pixels, the map decodes to {rows} x "
+                         f"{cols} patches of {h} x {w}")
+    precision = resolve_precision(dec)
+    if precision != residual.precision:
+        raise ValueError(f"the residual layer was made against a {residual.precision!r} decode, the decoder "
+                         f"runs {precision!r}: its base pixels would differ")
+    if residual.payload.device != code_map.device:
+        raise ValueError(f"the residual layer is on {residual.payload.device}, the map on {code_map.device}")
+    shape = (nr * h, nc * w, 3)
+    if out is None:
+        out = torch.empty(shape, dtype=torch.uint8, device=code_map.device)
+    elif tuple(out.shape) != shape or out.dtype != torch.uint8 or out.device != code_map.device \
+            or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous uint8 tensor of shape {shape} on {code_map.device}")
+    total = nr * nc
+    flags = torch.empty(total, dtype=torch.uint8, device=code_map.device)
+    for first in range(0, total, batch):
+        n = min(batch, total - first)
+        enc = E.embed_codemap(pq, code_map, (th, tw), r0, c0, nc, first, n)
+        P.decoder_forward_u8(dec, enc, mean, std, out, first, nc)
+        E.residual_apply(residual.payload, residual.offsets, residual.offsets_host, residual.adler, (rows, cols),
+                         (r0, c0, nc, first), out, (0, 0, nc, first), n, h, w, residual.max_error,
+                         flags[first:first + n])
+    bad = torch.nonzero(flags).flatten().cpu().tolist()
+    if bad:
+        fl = flags.cpu().tolist()
+        patches = [(r0 + i // nc, c0 + i % nc) for i in bad]
+        causes = [flag_causes(fl[i]) for i in bad]
+        shown = ", ".join(f"{p} {'/'.join(c)}" for p, c in zip(patches[:8], causes[:8]))
+        raise ResidualIntegrityError(f"residual layer: {len(patches)} patch(es) failed their checks at (row, col) "
+                                     f"{shown}{' ...' if len(patches) > 8 else ''}", out, flags.view(nr, nc),
+                                     patches, causes)
+    return out
 
 
 def tiles_to_map(tiles_u8: torch.Tensor, grid: Tuple[int, int]) -> torch.Tensor:

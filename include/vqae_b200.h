@@ -501,6 +501,58 @@ int vqae_pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int6
                     int64_t dst_r0, int64_t dst_c0, int64_t dst_region_cols, int64_t dst_first,
                     void* scratch, size_t scratch_bytes, void* stream);
 
+/* ---- near-lossless residual layer of stored code maps (csrc/residual.cu, DESIGN.md 4.15) ----------
+ * Patches are height x width x 3 uint8, n = 3 height width bytes in canvas order (row-major, channel
+ * innermost); x the original, base the decode of the map, e = max_error in [0, 127], d = x - base:
+ *   e = 0:  symbol s = d & 255,  x' = (base + s) & 255 = x;
+ *   e >= 1: k = sign(d) floor((|d| + e) / (2e + 1)), s = k & 255, x' = clamp(base + k (2e + 1), 0, 255),
+ *           |x - x'| <= e.
+ * A chunk per patch: 256 x u16 frequencies (total 2^14), 32 x u32 lane word counts, 32 x u32 final lane
+ * states, then the 16-bit words of lanes 0 .. 31 in decoder order, little-endian; symbol i is coded by rANS
+ * lane i mod 32 (32-bit state, L = 2^16, at most one word per symbol); 768 + 2 sum(w) bytes, at most
+ * 768 + 2 n.  Adler-32 values are zlib.adler32 of a patch's bytes in canvas order, (B << 16) | A.
+ * Every canvas is uint8 [rows, cols, 3] with the addressing tuple of vqae_quality_u8.
+ *
+ * vqae_residual_stats      hist[batch][256] (int64): exact symbol counts per patch; adler[batch][2]: the
+ *                          Adler-32 of base and of x'.
+ * vqae_residual_tables     freq[batch][256] (int32) from hist: packing.quantise_frequencies with S = 14.
+ * vqae_residual_encode     codes each patch of the call with its row of freq into offsets[batch + 1] and
+ *                          the payload (payload_capacity >= batch (768 + 2 n)).  A patch with a symbol of
+ *                          frequency 0 (freq not made from these pixels) gets a 0-byte chunk.
+ * vqae_residual_apply      decodes the chunks of patches (layer_r0 + q / layer_region_cols) grid_cols +
+ *                          layer_c0 + q % layer_region_cols, q = layer_first + t, of a layer of grid_rows x
+ *                          grid_cols patches and replaces the base pixels of patch t of the canvas with x'
+ *                          in place; adler holds the layer's [P][2] stored values.  flags[batch]: bit 0 the
+ *                          chunk failed (a lane not back at L with its words exactly consumed, a table not
+ *                          summing to 2^14, a length that disagrees with the word counts), bit 1 the base
+ *                          Adler differs, bit 2 the output Adler differs.  Reads of a chunk stay inside its
+ *                          own [offsets[p], offsets[p + 1]) range clamped to the payload.
+ * Integer arithmetic, no atomics: bitwise reproducible, independent of the batch and the grid.  Checked
+ * before anything is launched: VQAE_ERR_BAD_ARG for a null pointer, a non-positive extent, a negative e or
+ * first, a placement outside a canvas or the layer grid, a short payload_capacity, or offsets_host (the
+ * P + 1 offsets on the host) not starting at 0, ending at payload_bytes and stepping by an even
+ * 768 .. 768 + 2 n; VQAE_ERR_UNSUPPORTED for e > 127, height x width > 2^20 or first + batch > 2^31;
+ * VQAE_ERR_SCRATCH when scratch is missing or smaller than vqae_residual_encode_scratch_bytes.        */
+int vqae_residual_stats(const uint8_t* x, int64_t x_rows, int64_t x_cols, int64_t x_r0, int64_t x_c0,
+                        int64_t x_region_cols, int64_t x_first, const uint8_t* base, int64_t base_rows,
+                        int64_t base_cols, int64_t base_r0, int64_t base_c0, int64_t base_region_cols,
+                        int64_t base_first, int64_t batch, int height, int width, int max_error, int64_t* hist,
+                        uint32_t* adler, void* stream);
+int vqae_residual_tables(const int64_t* hist, int64_t batch, int32_t* freq, void* stream);
+size_t vqae_residual_encode_scratch_bytes(int64_t batch, int height, int width);
+int vqae_residual_encode(const uint8_t* x, int64_t x_rows, int64_t x_cols, int64_t x_r0, int64_t x_c0,
+                         int64_t x_region_cols, int64_t x_first, const uint8_t* base, int64_t base_rows,
+                         int64_t base_cols, int64_t base_r0, int64_t base_c0, int64_t base_region_cols,
+                         int64_t base_first, int64_t batch, int height, int width, int max_error,
+                         const int32_t* freq, int64_t* offsets, uint8_t* payload, int64_t payload_capacity,
+                         void* scratch, size_t scratch_bytes, void* stream);
+int vqae_residual_apply(const uint8_t* payload, int64_t payload_bytes, const int64_t* offsets_host,
+                        const int64_t* offsets, const uint32_t* adler, int64_t grid_rows, int64_t grid_cols,
+                        int64_t layer_r0, int64_t layer_c0, int64_t layer_region_cols, int64_t layer_first,
+                        uint8_t* canvas, int64_t rows, int64_t cols, int64_t r0, int64_t c0, int64_t region_cols,
+                        int64_t first, int64_t batch, int height, int width, int max_error, uint8_t* flags,
+                        void* stream);
+
 /* ---- f-4  training-mode codebook maintenance (layers/vq.py:47-94) -----------------------------
  * EMAVectorQuantizer._update_ema / _init_ema without the N x K one-hot matrix of the reference:
  *   vqae_ema_accumulate_f32   counts[k] = #{n : idx[n] = k},  dw[k,:] = sum of z[n,:] over those n
