@@ -129,6 +129,10 @@ SIGNATURES = {
     "vqae_pyramid_u8_scratch_bytes": (_sz, [_i64, _i, _i, _i]),
     "vqae_pyramid_u8": (_i, [_vp, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i, _i, _i, _vp, _vp, _vp, _i64, _i64,
                              _i64, _i64, _vp, _sz, _vp]),
+    "vqae_jpeg_tiles_scratch_bytes": (_sz, [_i64, _i64, _i, _i, _i64, _i64, _i, _i]),
+    "vqae_jpeg_tiles_worst_bytes": (_i64, [_i64, _i64, _i, _i, _i64, _i64, _i, _i]),
+    "vqae_jpeg_tiles": (_i, [_vp, _i64, _i64, _i64, _i, _i, _i64, _i64, _i, _i, _vp, _i, _vp, _vp, _vp, _i64, _vp,
+                             _sz, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

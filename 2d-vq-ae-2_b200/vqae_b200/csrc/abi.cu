@@ -596,6 +596,25 @@ int vqae_pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int6
                       scratch_bytes, (cudaStream_t)stream);
 }
 
+size_t vqae_jpeg_tiles_scratch_bytes(int64_t ext_h, int64_t ext_w, int tile, int overlap, int64_t row0,
+                                     int64_t nrows, int subsampling, int header_len) {
+    return jpeg_tiles_scratch_bytes(ext_h, ext_w, tile, overlap, row0, nrows, subsampling, header_len);
+}
+
+int64_t vqae_jpeg_tiles_worst_bytes(int64_t ext_h, int64_t ext_w, int tile, int overlap, int64_t row0,
+                                    int64_t nrows, int subsampling, int header_len) {
+    return jpeg_tiles_worst_bytes(ext_h, ext_w, tile, overlap, row0, nrows, subsampling, header_len);
+}
+
+int vqae_jpeg_tiles(const uint8_t* canvas, int64_t pitch, int64_t ext_h, int64_t ext_w, int tile, int overlap,
+                    int64_t row0, int64_t nrows, int quality, int subsampling, const uint8_t* headers_host,
+                    int header_len, const uint16_t* qtables_host, int64_t* offsets, uint8_t* payload,
+                    int64_t payload_capacity, void* scratch, size_t scratch_bytes, void* stream) {
+    return jpeg_tiles(canvas, pitch, ext_h, ext_w, tile, overlap, row0, nrows, quality, subsampling, headers_host,
+                      header_len, qtables_host, offsets, payload, payload_capacity, scratch, scratch_bytes,
+                      (cudaStream_t)stream);
+}
+
 int vqae_residual_stats(const uint8_t* x, int64_t x_rows, int64_t x_cols, int64_t x_r0, int64_t x_c0,
                         int64_t x_region_cols, int64_t x_first, const uint8_t* base, int64_t base_rows,
                         int64_t base_cols, int64_t base_r0, int64_t base_c0, int64_t base_region_cols,

@@ -22,7 +22,7 @@ STAMP = PKG / ".libvqae_b200.stamp"
 SOURCES = ["abi.cu", "conv_f32.cu", "stems.cu", "quantize.cu", "quantize_tc.cu", "tc_kernels.cu",
            "tc_down.cu", "tc_chain.cu", "tc_resident.cu", "up_tail.cu", "up_head.cu", "pack.cu",
            "mma_same.cu", "mma_down.cu", "mma_up.cu", "tc_split.cu", "mma_front.cu", "mma_stem.cu", "tc_down128.cu", "mma_same_split.cu", "ema.cu", "mbconv.cu",
-           "quality.cu", "codemap_pack.cu", "pyramid.cu", "residual.cu"]
+           "quality.cu", "codemap_pack.cu", "pyramid.cu", "residual.cu", "jpeg.cu"]
 # test / measurement aids: a separate library that links against the product library
 AID_SOURCES = ["testaids.cu", "tc_bench.cu"]
 AIDS_PATH = PKG / "libvqae_b200_testaids.so"

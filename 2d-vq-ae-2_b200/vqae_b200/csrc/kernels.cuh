@@ -221,4 +221,14 @@ int pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int64_t s
                int64_t dst_c0, int64_t dst_rc, int64_t dst_first, void* scratch, size_t scratch_bytes,
                cudaStream_t stream);
 
+// jpeg.cu (baseline JPEG tiles of a uint8 RGB canvas level)
+size_t jpeg_tiles_scratch_bytes(int64_t ext_h, int64_t ext_w, int tile, int overlap, int64_t row0, int64_t nrows,
+                                int subsampling, int header_len);
+int64_t jpeg_tiles_worst_bytes(int64_t ext_h, int64_t ext_w, int tile, int overlap, int64_t row0, int64_t nrows,
+                               int subsampling, int header_len);
+int jpeg_tiles(const uint8_t* canvas, int64_t pitch, int64_t ext_h, int64_t ext_w, int tile, int overlap,
+               int64_t row0, int64_t nrows, int quality, int subsampling, const uint8_t* headers_host,
+               int header_len, const uint16_t* qtables_host, int64_t* offsets, uint8_t* payload,
+               int64_t payload_capacity, void* scratch, size_t scratch_bytes, cudaStream_t stream);
+
 }  // namespace vqae

@@ -1029,6 +1029,40 @@ def pyramid_u8(src_canvas: Tensor, src_addr: Tuple[int, int, int, int], batch: i
                                 ws.numel(), _stream(dev)), "vqae_pyramid_u8")
 
 
+def jpeg_tiles(canvas: Tensor, tile: int, overlap: int, row0: int, nrows: int, quality: int, subsampling: int,
+               headers: bytes, qtables: np.ndarray) -> Tuple[Tensor, np.ndarray]:
+    """Baseline JPEG files of the tile rows [row0, row0 + nrows) of a uint8 RGB canvas level (vqae_jpeg_tiles):
+    ``canvas`` uint8 [H, W, 3] on a CUDA device with packed pixels (stride (pitch, 3, 1)); ``headers`` the 16
+    class headers of ``jpeg.level_headers``, ``qtables`` uint16 [2, 64] in zigzag order.  Returns
+    (payload uint8 on the device, trimmed to the files, offsets int64 [nrows * cols + 1] on the host)."""
+    lib = L.load()
+    require_cuda(canvas, "jpeg_tiles")
+    if canvas.dtype != torch.uint8 or canvas.dim() != 3 or canvas.shape[2] != 3 or canvas.stride(2) != 1 or \
+            canvas.stride(1) != 3:
+        raise ValueError("jpeg_tiles reads a uint8 [H, W, 3] canvas with packed pixels (strides (pitch, 3, 1))")
+    h, w = int(canvas.shape[0]), int(canvas.shape[1])
+    n_hdr = len(headers) // 16
+    if n_hdr * 16 != len(headers) or n_hdr == 0:
+        raise ValueError("headers must be 16 headers of one length")
+    qt = np.ascontiguousarray(qtables, dtype=np.uint16)
+    hb = np.frombuffer(headers, dtype=np.uint8)
+    args = (h, w, tile, overlap, row0, nrows, subsampling, n_hdr)
+    worst = lib.vqae_jpeg_tiles_worst_bytes(*args)
+    if worst < 0:
+        L.check(lib.vqae_jpeg_tiles(None, 0, h, w, tile, overlap, row0, nrows, quality, subsampling, None, n_hdr,
+                                    None, None, None, 0, None, 0, None), "vqae_jpeg_tiles")
+    dev = canvas.device
+    ncols = -(-w // tile)
+    offsets = torch.empty(nrows * ncols + 1, dtype=torch.int64, device=dev)
+    payload = torch.empty(worst, dtype=torch.uint8, device=dev)
+    ws = workspace(dev, lib.vqae_jpeg_tiles_scratch_bytes(*args))
+    L.check(lib.vqae_jpeg_tiles(_ptr(canvas), canvas.stride(0), h, w, tile, overlap, row0, nrows, quality,
+                                subsampling, hb.ctypes.data, n_hdr, qt.ctypes.data, _ptr(offsets), _ptr(payload),
+                                worst, _ptr(ws), ws.numel(), _stream(dev)), "vqae_jpeg_tiles")
+    offsets_host = offsets.cpu().numpy()
+    return payload[:int(offsets_host[-1])].clone(), offsets_host
+
+
 RESIDUAL_HEADER_BYTES = 768        # 256 x u16 frequencies, 32 x u32 word counts, 32 x u32 final states
 
 

@@ -496,6 +496,90 @@ def decompress_region_exact(model, code_map: torch.Tensor, code_hw: Tuple[int, i
     return out
 
 
+@torch.no_grad()
+def export_deepzoom(model, code_map: torch.Tensor, code_hw: Tuple[int, int], out_dir, name: str, tile: int = 254,
+                    overlap: int = 1, quality: int = 90, subsampling: int = 2, batch: int = 256, mean=None,
+                    std=None, band_pixels: int = 1 << 26) -> Dict[str, object]:
+    """Write a stored code map as a DeepZoom pyramid of JPEG tiles: ``out_dir/name.dzi`` and
+    ``out_dir/name_files/<level>/<col>_<row>.jpeg`` (OpenSeadragon, QuPath, OpenSlide's DeepZoom server).
+
+    The map is decoded once (``decompress_region``, same checks, ``batch``, ``mean`` / ``std``).  Level L of
+    the W x H slide (``jpeg.dz_levels``) is, with f = 2^(M-L): the decoded slide for f = 1; its
+    ``slide_pyramid`` level (exact box means, rounded once) for the f = 2 .. 512 that divide the patch height
+    and width (every f up to the patch size for the power-of-two patches of the shipped models); and for
+    every coarser f ``PIL.Image.reduce(2)`` of the next finer level, so the coarsest levels are chained,
+    rounded once per halving.  Every level is JPEG-encoded on the GPU (``jpeg.encode_tiles``), each tile byte-identical to
+    Pillow's encode of the same crop at ``quality`` / ``subsampling``, ``band_pixels`` level pixels of
+    tile rows per call to bound the encoder's memory.  Returns the .dzi path, the level count, tile count,
+    total bytes and per-phase seconds (decode, pyramid, encode, write)."""
+    import time
+
+    from PIL import Image
+
+    from . import jpeg as JP
+    from .pyramid import slide_pyramid
+    JP.check_quality(quality, subsampling)
+    JP.check_tiling(tile, overlap)
+    if not name or "/" in name or name in (".", ".."):
+        raise ValueError(f"name {name!r} is not a file name")
+    if band_pixels <= 0:
+        raise ValueError("band_pixels must be positive")
+    secs = {"decode": 0.0, "pyramid": 0.0, "encode": 0.0, "write": 0.0}
+
+    def sync_time(key, t0):
+        torch.cuda.synchronize(code_map.device)
+        secs[key] += time.perf_counter() - t0
+
+    t0 = time.perf_counter()
+    slide = decompress_region(model, code_map, code_hw, batch=batch, mean=mean, std=std)
+    sync_time("decode", t0)
+    dev = slide.device
+    ph, pw = (int(v) * P.patch_scale(model.decoder) for v in code_hw)
+    height, width = int(slide.shape[0]), int(slide.shape[1])
+    dims = JP.dz_levels(width, height)
+    m = len(dims) - 1
+    t0 = time.perf_counter()
+    gpu_factors = [1 << k for k in range(1, min(m, 9) + 1) if ph % (1 << k) == 0 and pw % (1 << k) == 0]
+    levels = {1: slide}
+    if gpu_factors:
+        levels.update(slide_pyramid(slide, (ph, pw), gpu_factors))
+    sync_time("pyramid", t0)
+    out_dir = Path(out_dir)
+    files = out_dir / f"{name}_files"
+    n_tiles, n_bytes, finer = 0, 0, None
+    for lv in range(m, -1, -1):
+        f = 1 << (m - lv)
+        w_l, h_l = dims[lv]
+        if f in levels:
+            canvas = levels.pop(f)
+        else:                                                  # chained on the host from the next finer level
+            t0 = time.perf_counter()
+            canvas = torch.from_numpy(np.array(Image.fromarray(finer).reduce(2))).to(dev)
+            sync_time("pyramid", t0)
+        assert tuple(canvas.shape) == (h_l, w_l, 3)
+        finer = canvas.cpu().numpy() if f * 2 not in levels and lv > 0 else None
+        cols, rows = JP.tile_grid(w_l, h_l, tile)
+        band = max(1, band_pixels // (w_l * min(h_l, tile + 2 * overlap)))
+        level_dir = files / str(lv)
+        level_dir.mkdir(parents=True, exist_ok=True)
+        for r0 in range(0, rows, band):
+            t0 = time.perf_counter()
+            tiles = JP.encode_tiles(canvas, tile, overlap, quality, subsampling, rows=(r0, min(band, rows - r0)))
+            host = tiles.payload.cpu().numpy()
+            sync_time("encode", t0)
+            t0 = time.perf_counter()
+            for r in range(r0, r0 + tiles.grid[1]):
+                for c in range(cols):
+                    (level_dir / f"{c}_{r}.jpeg").write_bytes(tiles.tile_bytes(c, r, host))
+            secs["write"] += time.perf_counter() - t0
+            n_tiles += cols * tiles.grid[1]
+            n_bytes += tiles.nbytes()
+        del canvas
+    dzi = out_dir / f"{name}.dzi"
+    dzi.write_text(JP.dzi_xml(width, height, tile, overlap))
+    return {"dzi": dzi, "levels": m + 1, "tiles": n_tiles, "bytes": n_bytes, "seconds": secs}
+
+
 def tiles_to_map(tiles_u8: torch.Tensor, grid: Tuple[int, int]) -> torch.Tensor:
     """[P,th,tw] tiles in row-major patch order -> [rows*th, cols*tw] map (pure view ops)."""
     rows, cols = grid

@@ -501,6 +501,33 @@ int vqae_pyramid_u8(const uint8_t* src, int64_t src_rows, int64_t src_cols, int6
                     int64_t dst_r0, int64_t dst_c0, int64_t dst_region_cols, int64_t dst_first,
                     void* scratch, size_t scratch_bytes, void* stream);
 
+/* ---- baseline JPEG tiles of a uint8 RGB canvas level (csrc/jpeg.cu, DESIGN.md 4.16) ---------------------
+ * The level is ext_h x ext_w pixels of the canvas uint8 [.., pitch] (row y, column x, channel ch at
+ * canvas[y * pitch + 3 x + ch]).  With tile size `tile` and `overlap`, tile (c, r) covers x in
+ * [max(0, c tile - overlap), min(ext_w, (c + 1) tile + overlap)) and likewise y; the call encodes the tile
+ * rows [row0, row0 + nrows), every column, row-major.  Each tile becomes the baseline JFIF file libjpeg
+ * writes for quality `quality` and subsampling 0 (4:4:4) or 2 (4:2:0) with the standard Huffman tables:
+ * headers_host (host) holds 16 headers of header_len bytes, header (4 row class + column class) for the
+ * tiles of that class (class 0: the first row / column, 1: the middle ones, 2: the second-to-last, 3: the
+ * last; in a grid of n < 4 tiles the lower class of a tile that is several); qtables_host (host)
+ * the luminance and chrominance tables of that quality, 2 x 64 in zigzag order as in the DQT segments.
+ * The files go back to back into `payload`, file i at [offsets[i], offsets[i + 1]) (offsets: device,
+ * nrows * ncols + 1 int64, offsets[0] = 0).  Integer arithmetic, no atomics: each file depends on its
+ * pixels, the tables and the subsampling only.  Checked before anything is launched: VQAE_ERR_BAD_ARG for
+ * a null pointer, a non-positive extent, tile <= 0, overlap < 0, overlap >= tile, rows outside the tile
+ * grid, pitch < 3 ext_w, a table entry outside [1, 255] or payload_capacity < vqae_jpeg_tiles_worst_bytes;
+ * VQAE_ERR_UNSUPPORTED for quality outside 1 .. 100, subsampling not 0 or 2, or a tile side over 65535;
+ * VQAE_ERR_SCRATCH when scratch_bytes < vqae_jpeg_tiles_scratch_bytes.  The two size queries return 0 /
+ * -1 for arguments the encoder rejects.                                                                */
+size_t vqae_jpeg_tiles_scratch_bytes(int64_t ext_h, int64_t ext_w, int tile, int overlap, int64_t row0,
+                                     int64_t nrows, int subsampling, int header_len);
+int64_t vqae_jpeg_tiles_worst_bytes(int64_t ext_h, int64_t ext_w, int tile, int overlap, int64_t row0,
+                                    int64_t nrows, int subsampling, int header_len);
+int vqae_jpeg_tiles(const uint8_t* canvas, int64_t pitch, int64_t ext_h, int64_t ext_w, int tile, int overlap,
+                    int64_t row0, int64_t nrows, int quality, int subsampling, const uint8_t* headers_host,
+                    int header_len, const uint16_t* qtables_host, int64_t* offsets, uint8_t* payload,
+                    int64_t payload_capacity, void* scratch, size_t scratch_bytes, void* stream);
+
 /* ---- near-lossless residual layer of stored code maps (csrc/residual.cu, DESIGN.md 4.15) ----------
  * Patches are height x width x 3 uint8, n = 3 height width bytes in canvas order (row-major, channel
  * innermost); x the original, base the decode of the map, e = max_error in [0, 127], d = x - base:
